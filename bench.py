@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- verified signature-sets/s of verify_multiple_aggregate_signatures on B200.
 
-Contract (see the task statement):  python bench.py --gpus N --steps K --warmup W [--impl reference]
+Usage:  python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
   * workload at N = 1: BASELINE.json configs[3] -- 8192 attestation sets x 128 public keys, distinct random
     32-byte messages, 63-bit batch scalars (C4).  For N > 1 every rank keeps 8192 sets (weak scaling), so N = 8
     is BASELINE.json configs[4] (2^16 sets, NCCL combine of the 592-byte partial Miller products).
@@ -252,8 +252,13 @@ def main():
     ap.add_argument("--h2c-msgs", type=int, default=65536, help="messages per hash_to_G2 batch of the second metric")
     ap.add_argument("--no-next-rows", action="store_true", help="skip the SURVEY 8(f) rows (decompression, aggregation, per-item verification)")
     ap.add_argument("--breakdown", action="store_true", help="print the per-stage device times to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last headline step and the last hash_to_G2 batch returned as DIR/<name>.npy "
+                         "(float32 / float64; fixed inputs, so two builds can be compared output for output)")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("bench.py: --dump-outputs dumps the GPU path; the reference arm has no outputs to dump")
         return reference_main(args)
 
     import numpy as np
@@ -585,7 +590,7 @@ def _bench_lanes(eng, comm, table, lanes, setup, args, world, rank, local_rank, 
             assert r[0] and r[1] == -1, "verification of the valid synthetic batch must accept"
         with stage_lock:
             st = {k: v / (steps * len(use_lanes)) for k, v in stage_acc.items()}
-        return float(t.item()), total_launches() - launches0, st, res[-1]
+        return float(t.item()), total_launches() - launches0, st, res[-len(use_lanes):]      # results of the last step
 
     W = max(args.warmup, 3)
     K = args.steps
@@ -841,12 +846,29 @@ def _bench_lanes(eng, comm, table, lanes, setup, args, world, rank, local_rank, 
                           "cpu_baseline": cpu_h2c},
            "next_rows": next_rows,
            "gpu_launches": launches, "clocks": clocks, "roofline": roofline, "cpu_baseline": cpu,
-           "accept": bool(last[0]),
+           "accept": bool(last[-1][0]),
            "ms_per_step_by_rank": by_rank if world > 1 else None,
            "checks": "valid batch: same GT on every rank and for both key forms; tampered message on the last rank: reject on every rank with one GT; non-subgroup signature on the last rank: global first_bad on every rank"}
     if args.breakdown:
         print(json.dumps({"overlapped": stages, "serialised": stages_serial, "pipelined": stages_pipe}, indent=1), file=sys.stderr)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, hout.cpu().numpy().reshape(nh, 192))
     print(json.dumps(out), flush=True)
+
+
+def dump_outputs(out_dir, last_step, h2c_points):
+    """What a caller of the timed paths received, as float arrays (bytes 0..255 and small integers are exact):
+    verify_*: one row per call of the last headline step (accept, first_bad and, at N = 1, the 576 GT bytes);
+    hash_to_g2: the 192-byte wire points of every (n // 4096)-th of the n messages of the last batch, at most 4096 of them."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"verify_accept": np.array([r[0] for r in last_step], dtype=np.float32),
+              "verify_first_bad": np.array([r[1] for r in last_step], dtype=np.float64),
+              "hash_to_g2": h2c_points[::max(1, len(h2c_points) // 4096)][:4096].astype(np.float32)}
+    if len(last_step[0]) == 3:
+        arrays["verify_gt"] = np.stack([np.frombuffer(r[2], dtype=np.uint8) for r in last_step]).astype(np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 if __name__ == "__main__":
