@@ -43,7 +43,7 @@ B3_FN void coop_mul_p1(coop_ws& ws, const fp12& a, const fp12& b, int tid) {
         fp_add(B1, y.c0, y.c1);
     }
     fp u2, v1, v2;
-    fp_neg(u2, x.c1);
+    fp_neg_nr(u2, x.c1);                           // <= 2p: an operand of the dual product only
     fp_select(u2, comp != 0, x.c1, u2);
     fp_select(v1, comp != 0, B1, B0);
     fp_select(v2, comp != 0, B0, B1);
@@ -148,7 +148,7 @@ B3_FN void coop_mul_line_p1(coop_ws& ws, const fp12& a, const fp12& l, int tid) 
         fp_add(B1, y.c0, y.c1);
     }
     fp u2, v1, v2;
-    fp_neg(u2, x.c1);
+    fp_neg_nr(u2, x.c1);                           // <= 2p: an operand of the dual product only
     fp_select(u2, comp != 0, x.c1, u2);
     fp_select(v1, comp != 0, B1, B0);
     fp_select(v2, comp != 0, B0, B1);

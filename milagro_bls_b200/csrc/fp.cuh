@@ -3,8 +3,11 @@
 // Replaces (does not port) the reference's FP/Big/DBig layer:
 //   /root/reference/incubator-milagro-crypto-rust/src/fp.rs:306-314,390-398 (mul/sqr -> Big::mul + Big::monty)
 //   /root/reference/incubator-milagro-crypto-rust/src/big.rs:950-986,1064-1106 (7 x 58-bit limbs, R = 2^406)
-// The reference's radix and lazy-reduction bookkeeping are not observable (SURVEY.md B.1); here every
-// value is kept fully reduced in [0, p).
+// The reference's radix and lazy-reduction bookkeeping are not observable (SURVEY.md B.1).  Here every device value
+// is a Montgomery residue in [0, 2p), not necessarily the canonical one: p < 2^381 leaves three spare bits under R, so a
+// product of two such values, (ab + mp)/R < 4p^2/R + p < 1.41p, needs no final subtraction, and additions and subtractions
+// reduce modulo 2p.  The canonical representative (fp_canon) is formed only where a value is compared, tested for zero,
+// has its sign or parity read, or leaves the device: fp_is_zero, fp_eq, fp_from_mont, fp_inv and the wire writers.
 //
 // The multiplier is a row-wise Montgomery product with two 32-bit-staggered accumulators ("even"/"odd"
 // columns) so that every 32x32->64 partial product is one `mad.lo.cc`/`madc.hi.cc` pair on an aligned
@@ -102,17 +105,12 @@ B3_FN void madc_wide_last(uint32_t& lo, uint32_t& hi, uint32_t a, uint32_t b) {
 // ------------------------------------------------------------------------------------------------
 // basic predicates / moves
 // ------------------------------------------------------------------------------------------------
+// a == 0 mod p for a in [0, 2p): a is 0 or p
 B3_FN bool fp_is_zero(const fp& a) {
-    uint32_t t = 0;
+    uint32_t z = 0, q = 0;
 #pragma unroll
-    for (int i = 0; i < 12; i++) t |= a.l[i];
-    return t == 0;
-}
-B3_FN bool fp_eq(const fp& a, const fp& b) {
-    uint32_t t = 0;
-#pragma unroll
-    for (int i = 0; i < 12; i++) t |= a.l[i] ^ b.l[i];
-    return t == 0;
+    for (int i = 0; i < 12; i++) { z |= a.l[i]; q |= a.l[i] ^ FP_P.l[i]; }
+    return z == 0 || q == 0;
 }
 // r = c ? a : b
 B3_FN void fp_select(fp& r, bool c, const fp& a, const fp& b) {
@@ -124,24 +122,26 @@ B3_FN void fp_set(fp& r, const fp& a) {
     for (int i = 0; i < 12; i++) r.l[i] = a.l[i];
 }
 
-// t (in [0, 2p)) -> r in [0, p)
-B3_FN void fp_final_sub(fp& r, const uint32_t* t) {
+// r = t < m ? t : t - m      (m = p or 2p)
+B3_FN void fp_cond_sub(fp& r, const uint32_t* t, const fp& m) {
     uint32_t s[12];
-    s[0] = sub_cc(t[0], FP_P.l[0]);
+    s[0] = sub_cc(t[0], m.l[0]);
 #pragma unroll
-    for (int i = 1; i < 12; i++) s[i] = subc_cc(t[i], FP_P.l[i]);
-    uint32_t borrow = subc(0, 0);          // 0xffffffff if t < p
+    for (int i = 1; i < 12; i++) s[i] = subc_cc(t[i], m.l[i]);
+    uint32_t borrow = subc(0, 0);          // 0xffffffff if t < m
 #pragma unroll
     for (int i = 0; i < 12; i++) r.l[i] = borrow ? t[i] : s[i];
 }
+// a in [0, 2p) -> the canonical representative in [0, p)
+B3_FN void fp_canon(fp& r, const fp& a) { fp_cond_sub(r, a.l, FP_P); }
 
 B3_FN void fp_add(fp& r, const fp& a, const fp& b) {
     uint32_t t[12];
     t[0] = add_cc(a.l[0], b.l[0]);
 #pragma unroll
     for (int i = 1; i < 11; i++) t[i] = addc_cc(a.l[i], b.l[i]);
-    t[11] = addc(a.l[11], b.l[11]);        // a + b < 2p < 2^384: no carry out
-    fp_final_sub(r, t);
+    t[11] = addc(a.l[11], b.l[11]);        // a + b < 4p < 2^384: no carry out
+    fp_cond_sub(r, t, FP_2P);
 }
 
 B3_FN void fp_sub(fp& r, const fp& a, const fp& b) {
@@ -149,41 +149,68 @@ B3_FN void fp_sub(fp& r, const fp& a, const fp& b) {
     t[0] = sub_cc(a.l[0], b.l[0]);
 #pragma unroll
     for (int i = 1; i < 12; i++) t[i] = subc_cc(a.l[i], b.l[i]);
-    uint32_t m = subc(0, 0);               // all-ones if a < b
-    r.l[0] = add_cc(t[0], FP_P.l[0] & m);
+    uint32_t m = subc(0, 0);               // all-ones if a < b: a - b + 2p in (0, 2p)
+    r.l[0] = add_cc(t[0], FP_2P.l[0] & m);
 #pragma unroll
-    for (int i = 1; i < 11; i++) r.l[i] = addc_cc(t[i], FP_P.l[i] & m);
-    r.l[11] = addc(t[11], FP_P.l[11] & m);
+    for (int i = 1; i < 11; i++) r.l[i] = addc_cc(t[i], FP_2P.l[i] & m);
+    r.l[11] = addc(t[11], FP_2P.l[11] & m);
 }
 
+B3_FN bool fp_eq(const fp& a, const fp& b) {
+    fp d;
+    fp_sub(d, a, b);
+    return fp_is_zero(d);
+}
+
+// r = 2p - a, and 0 for a = 0 (so that the result stays below 2p)
 B3_FN void fp_neg(fp& r, const fp& a) {
-    bool z = fp_is_zero(a);
+    uint32_t z = 0;
+#pragma unroll
+    for (int i = 0; i < 12; i++) z |= a.l[i];
     uint32_t t[12];
-    t[0] = sub_cc(FP_P.l[0], a.l[0]);
+    t[0] = sub_cc(FP_2P.l[0], a.l[0]);
 #pragma unroll
-    for (int i = 1; i < 11; i++) t[i] = subc_cc(FP_P.l[i], a.l[i]);
-    t[11] = subc(FP_P.l[11], a.l[11]);
+    for (int i = 1; i < 11; i++) t[i] = subc_cc(FP_2P.l[i], a.l[i]);
+    t[11] = subc(FP_2P.l[11], a.l[11]);
 #pragma unroll
-    for (int i = 0; i < 12; i++) r.l[i] = z ? 0u : t[i];
+    for (int i = 0; i < 12; i++) r.l[i] = z == 0 ? 0u : t[i];
 }
 
 B3_FN void fp_dbl(fp& r, const fp& a) { fp_add(r, a, a); }
 
-// r = a/2 mod p
+// Unreduced forms, for an operand that goes straight into a product and nowhere else (see fp_mul_inl for the bounds):
+// r = a + b < 4p, and r = 2p - a in (0, 2p].
+B3_FN void fp_add_nr(fp& r, const fp& a, const fp& b) {
+    r.l[0] = add_cc(a.l[0], b.l[0]);
+#pragma unroll
+    for (int i = 1; i < 11; i++) r.l[i] = addc_cc(a.l[i], b.l[i]);
+    r.l[11] = addc(a.l[11], b.l[11]);
+}
+B3_FN void fp_neg_nr(fp& r, const fp& a) {
+    r.l[0] = sub_cc(FP_2P.l[0], a.l[0]);
+#pragma unroll
+    for (int i = 1; i < 11; i++) r.l[i] = subc_cc(FP_2P.l[i], a.l[i]);
+    r.l[11] = subc(FP_2P.l[11], a.l[11]);
+}
+
+// r = a/2 mod p: (a + p)/2 < 1.5p for odd a, a/2 < p for even a
 B3_FN void fp_half(fp& r, const fp& a) {
     uint32_t m = 0u - (a.l[0] & 1u);
     uint32_t t[12];
     t[0] = add_cc(a.l[0], FP_P.l[0] & m);
 #pragma unroll
     for (int i = 1; i < 11; i++) t[i] = addc_cc(a.l[i], FP_P.l[i] & m);
-    t[11] = addc(a.l[11], FP_P.l[11] & m);  // < 2p < 2^384
+    t[11] = addc(a.l[11], FP_P.l[11] & m);  // < 3p < 2^384
 #pragma unroll
     for (int i = 0; i < 11; i++) r.l[i] = (t[i] >> 1) | (t[i + 1] << 31);
     r.l[11] = t[11] >> 1;
 }
 
 // ------------------------------------------------------------------------------------------------
-// Montgomery multiplication  r = a * b / 2^384 mod p      (a < p required; b any 384-bit value)
+// Montgomery multiplication  r = a * b / 2^384 mod p, r < 2p      (a, b <= 2p; or a < 4p and b < 2p; or a < p and b any
+// 384-bit value).  The running value of the row-wise reduction stays below a + p < 5p < 2^384, so the two 12-limb
+// accumulators do not overflow; the result (ab + mp)/2^384 < 8p^2/2^384 + p < 1.82p (or < p + p for the last form) needs
+// no final subtraction.
 // ------------------------------------------------------------------------------------------------
 // acc[0..11] = sum_{j even} x[j] * y * 2^(32 j)            (no carries: products do not overlap)
 B3_FN void b3_mul_row(uint32_t* acc, const uint32_t* x, uint32_t y) {
@@ -228,16 +255,16 @@ B3_FN void fp_mul_inl(fp& r, const fp& a, const fp& b) {
         b3_mont_row(even, odd, av, bv[i], i == 0);
         b3_mont_row(odd, even, av, bv[i + 1], false);
     }
-    even[0] = add_cc(even[0], odd[1]);
+    r.l[0] = add_cc(even[0], odd[1]);
 #pragma unroll
-    for (int i = 1; i < 11; i++) even[i] = addc_cc(even[i], odd[i + 1]);
-    even[11] = addc(even[11], 0);
-    fp_final_sub(r, even);
+    for (int i = 1; i < 11; i++) r.l[i] = addc_cc(even[i], odd[i + 1]);
+    r.l[11] = addc(even[11], 0);
 }
 
-// Dual product with ONE reduction:  r = (a1*b1 + a2*b2) / 2^384 mod p      (a1, a2, b1, b2 < p)
-// 2 x 144 + 156 multiply-accumulates instead of 2 x 300.  The running value stays below 3p(1 + 2^-32) < 2^383, and the
-// result below p(1 + 2p/2^384) < 2p, so the accumulator shapes and the single final subtraction of fp_mul_inl carry over.
+// Dual product with ONE reduction:  r = (a1*b1 + a2*b2) / 2^384 mod p, r < 2p      (a1, a2 <= 2p; b1, b2 < 2p)
+// 2 x 144 + 156 multiply-accumulates instead of 2 x 300.  The running value stays below (a1 + a2 + p)(1 + 2^-32) < 5.01p
+// < 2^384 and the result below 8p^2/2^384 + p < 1.82p, so the accumulator shapes of fp_mul_inl carry over and there is no
+// final subtraction.
 B3_FN void b3_mont_row2(uint32_t* even, uint32_t* odd, const uint32_t* a1, uint32_t b1i, const uint32_t* a2, uint32_t b2i, bool first) {
     if (first) {
         b3_mul_row(odd, a1 + 1, b1i);
@@ -265,16 +292,16 @@ B3_FN void fp_mul2_inl(fp& r, const fp& a1, const fp& b1, const fp& a2, const fp
         b3_mont_row2(even, odd, a1v, b1v[i], a2v, b2v[i], i == 0);
         b3_mont_row2(odd, even, a1v, b1v[i + 1], a2v, b2v[i + 1], false);
     }
-    even[0] = add_cc(even[0], odd[1]);
+    r.l[0] = add_cc(even[0], odd[1]);
 #pragma unroll
-    for (int i = 1; i < 11; i++) even[i] = addc_cc(even[i], odd[i + 1]);
-    even[11] = addc(even[11], 0);
-    fp_final_sub(r, even);
+    for (int i = 1; i < 11; i++) r.l[i] = addc_cc(even[i], odd[i + 1]);
+    r.l[11] = addc(even[11], 0);
 }
-// Six-term dot product with ONE reduction:  r = (sum_{t<6} a[t] * b[t]) / 2^384 mod p     (all operands < p)
-// 6 x 144 + 156 = 1020 multiply-accumulates instead of 6 x 300 plus five additions.  Running value < 7p(1 + 2^-32)
-// < 2^384 and result < p(1 + 6p/2^384) < 1.61p, so the accumulators and the single final subtraction carry over
-// from fp_mul_inl.  Operands are read through pointers (they live in local/shared memory: Fp12 accumulators).
+// Six-term dot product with ONE reduction:  r = (sum_{t<6} a[t] * b[t]) / 2^384 mod p, r < 2p     (all operands < 2p)
+// 6 x 144 + 156 = 1020 multiply-accumulates instead of 6 x 300 plus five additions.  The running value is below
+// (sum a[t] + p)(1 + 2^-32): six operands below 2p would reach 13p > 2^384, so the a[t] are made canonical on load and it
+// stays below 7p(1 + 2^-32) < 2^384.  The result is below 12p^2/2^384 + p < 2.22p: one conditional subtraction of 2p.
+// Operands are read through pointers (they live in local/shared memory: Fp12 accumulators).
 struct fp_dot6_args {
     const fp* a[6];
     const fp* b[6];
@@ -285,6 +312,10 @@ B3_FN_NOINLINE void fp_dot6(fp& r, fp_dot6_args q) {
     for (int t = 0; t < 6; t++) {
 #pragma unroll
         for (int i = 0; i < 12; i++) av[t][i] = q.a[t]->l[i];
+        fp c;
+        fp_cond_sub(c, av[t], FP_P);
+#pragma unroll
+        for (int i = 0; i < 12; i++) av[t][i] = c.l[i];
     }
 #pragma unroll
     for (int i = 0; i < 12; i++) {
@@ -316,15 +347,17 @@ B3_FN_NOINLINE void fp_dot6(fp& r, fp_dot6_args q) {
 #pragma unroll
     for (int i = 1; i < 11; i++) even[i] = addc_cc(even[i], odd[i + 1]);
     even[11] = addc(even[11], 0);
-    fp_final_sub(r, even);
+    fp_cond_sub(r, even, FP_2P);
 }
 
 #if !defined(B3_HOSTSIM)
 // Register-resident dot product for the group-cooperative Miller accumulation (kernels.cuh, k_miller_accum): the `a`
 // operands are the caller's registers (Fp12 coefficients gathered by warp shuffles), the `b` operands are read from shared
-// memory four limbs at a time (LDS.128).  Same accumulator shapes and bounds as fp_dot6.
+// memory four limbs at a time (LDS.128).  Same accumulator shapes as fp_dot6.
 __device__ __forceinline__ uint32_t b3_u4_get(const uint4& v, int i) { return i == 0 ? v.x : i == 1 ? v.y : i == 2 ? v.z : v.w; }
-// Three terms, for the Karatsuba form of the sparse line product: 3 x 144 + 156 multiply-accumulates.
+// Three terms, for the Karatsuba form of the sparse line product: 3 x 144 + 156 multiply-accumulates.  All operands < 2p:
+// the running value stays below (a0 + a1 + a2 + p)(1 + 2^-32) < 7.01p < 2^384, the result below 12p^2/2^384 + p < 2.22p,
+// so it ends with one conditional subtraction of 2p.
 __device__ __forceinline__ void fp_dot3_rs(fp& r, const fp& a0, const fp& a1, const fp& a2, const fp* b0, const fp* b1, const fp* b2) {
     uint32_t even[12], odd[12];
     const fp* bp[3] = {b0, b1, b2};
@@ -366,7 +399,7 @@ __device__ __forceinline__ void fp_dot3_rs(fp& r, const fp& a0, const fp& a1, co
 #pragma unroll
     for (int i = 1; i < 11; i++) even[i] = addc_cc(even[i], odd[i + 1]);
     even[11] = addc(even[11], 0);
-    fp_final_sub(r, even);
+    fp_cond_sub(r, even, FP_2P);
 }
 #endif
 
@@ -380,14 +413,14 @@ __device__ __noinline__ fp fp_dot3_rs_v(fp a0, fp a1, fp a2, const fp* b0, const
 }
 #endif
 
-// Montgomery SQUARING  r = a^2 / 2^384 mod p  (a < p), row-wise with the same interleaved reduction as fp_mul_inl, but using
+// Montgomery SQUARING  r = a^2 / 2^384 mod p, r < 2p  (a < 2p), row-wise with the same interleaved reduction as fp_mul_inl, but using
 //   a^2 = sum_i a_i 2^(32 i) * ( a_i 2^(32 i) + 2 sum_{j>i} a_j 2^(32 j) ):
 // row i adds a_i times the limbs j >= i of that bracket only -- a_i itself at j = i, a_(i+1) << 1 at j = i + 1 and the limbs
-// d_j = (a_j << 1) | (a_(j-1) >> 31) of 2a above (2a < 2^382 has no 13th limb) -- i.e. 12 - i products instead of 12:
+// d_j = (a_j << 1) | (a_(j-1) >> 31) of 2a above (2a < 4p < 2^383 has no 13th limb) -- i.e. 12 - i products instead of 12:
 // 78 + 144 + 12 = 234 multiply-accumulates instead of 300.  Every contribution to limb k (pairs i + j = k) is added in a
 // row min(i, j) <= k, before limb k is reduced, so the interleaved reduction stays valid.  Bounds: the running value
-// obeys W' < W / 2^32 + 2a + p, hence W < 3p (1 + 2^-32) < 2^383 as in fp_mul2_inl (same accumulator shapes, same dropped
-// carries), and the result (a^2 + m p) / 2^384 < 1.11 p needs the one final subtraction.
+// obeys W' < W / 2^32 + 2a + p, hence W < 5p (1 + 2^-32) < 2^384 as in fp_mul2_inl (same accumulator shapes, same dropped
+// carries), and the result (a^2 + m p) / 2^384 < 4p^2/2^384 + p < 1.41p needs no final subtraction.
 template <int I>
 B3_FN void b3_sqr_row(uint32_t* E, uint32_t* O, const uint32_t* a, const uint32_t* d) {
 #define B3_SQW(j) ((j) == I ? a[(j)] : (j) == I + 1 ? (a[(j)] << 1) : d[(j)])
@@ -434,11 +467,10 @@ B3_FN void fp_sqr_inl(fp& r, const fp& a) {
     b3_sqr_row<6>(even, odd, av, d);  b3_sqr_row<7>(odd, even, av, d);
     b3_sqr_row<8>(even, odd, av, d);  b3_sqr_row<9>(odd, even, av, d);
     b3_sqr_row<10>(even, odd, av, d); b3_sqr_row<11>(odd, even, av, d);
-    even[0] = add_cc(even[0], odd[1]);
+    r.l[0] = add_cc(even[0], odd[1]);
 #pragma unroll
-    for (int i = 1; i < 11; i++) even[i] = addc_cc(even[i], odd[i + 1]);
-    even[11] = addc(even[11], 0);
-    fp_final_sub(r, even);
+    for (int i = 1; i < 11; i++) r.l[i] = addc_cc(even[i], odd[i + 1]);
+    r.l[11] = addc(even[11], 0);
 }
 
 // Out-of-line multipliers take and return their operands BY VALUE: ptxas then passes them in registers, and the
@@ -454,7 +486,8 @@ B3_FN void fp_sqr(fp& r, const fp& a) { r = fp_sqr_v(a); }
 
 // Montgomery form <-> canonical
 B3_FN void fp_to_mont(fp& r, const fp& a) { fp_mul(r, FP_R2, a); }       // a any 384-bit value
-B3_FN void fp_from_mont(fp& r, const fp& a) { fp_mul(r, a, FP_RAW_ONE); }
+// (a + mp)/2^384 <= p: only a residue of 0 (a = p) comes out non-canonical, as p
+B3_FN void fp_from_mont(fp& r, const fp& a) { fp t; fp_mul(t, a, FP_RAW_ONE); fp_canon(r, t); }
 
 // r = a^e for a fixed public exponent e (plain 384-bit integer): 5-bit SLIDING windows over a table of the odd powers
 // a, a^3, .., a^31 (one squaring + 15 multiplications), so a window is spent only on a bit string that starts and ends with
@@ -510,10 +543,11 @@ B3_FN bool fp_raw_is_one(const fp& a) {
 // 1/a mod p (0 -> 0) by the binary extended Euclidean algorithm on the Montgomery representative, about 5x fewer
 // instructions than the Fermat exponentiation a^(p-2) the reference uses (A/fp.rs:608-616); the value is the same.
 // With abar = a R: the loop yields abar^-1 = a^-1 R^-1 as a plain integer; one multiplication by R^3 gives a^-1 R.
-// Data-dependent control flow (the operand is public on this path).
+// Data-dependent control flow (the operand is public on this path).  The loop runs on the canonical representative.
 B3_FN_NOINLINE void fp_inv(fp& r, const fp& a) {
-    if (fp_is_zero(a)) { r = FP_NIL; return; }
-    fp u = a, v = FP_P, x1 = FP_RAW_ONE, x2 = FP_NIL;
+    fp u, v = FP_P, x1 = FP_RAW_ONE, x2 = FP_NIL;
+    fp_canon(u, a);
+    if (fp_is_zero(u)) { r = FP_NIL; return; }
     while (!fp_raw_is_one(u) && !fp_raw_is_one(v)) {
         if (!(u.l[0] & 1u)) {
 #pragma unroll
@@ -608,13 +642,16 @@ B3_FN void wire_store(uint8_t* out, const b3_q16* q) {
     for (int i = 0; i < N16; i++) reinterpret_cast<uint4*>(out)[i] = q[i];
 #endif
 }
-// 48 big-endian bytes held as three 16-byte words <-> raw limbs (limb i = byte-swapped word 11 - i)
+// 48 big-endian bytes held as three 16-byte words <-> raw limbs (limb i = byte-swapped word 11 - i); the writer takes a value
+// below 2p and emits its canonical representative
 B3_FN void fp_raw_from_q(fp& r, const b3_q16* q) {
     r.l[0] = b3_bswap(q[2].w); r.l[1] = b3_bswap(q[2].z); r.l[2] = b3_bswap(q[2].y); r.l[3] = b3_bswap(q[2].x);
     r.l[4] = b3_bswap(q[1].w); r.l[5] = b3_bswap(q[1].z); r.l[6] = b3_bswap(q[1].y); r.l[7] = b3_bswap(q[1].x);
     r.l[8] = b3_bswap(q[0].w); r.l[9] = b3_bswap(q[0].z); r.l[10] = b3_bswap(q[0].y); r.l[11] = b3_bswap(q[0].x);
 }
-B3_FN void fp_raw_to_q(b3_q16* q, const fp& a) {
+B3_FN void fp_raw_to_q(b3_q16* q, const fp& v) {
+    fp a;
+    fp_canon(a, v);
     q[2].w = b3_bswap(a.l[0]); q[2].z = b3_bswap(a.l[1]); q[2].y = b3_bswap(a.l[2]); q[2].x = b3_bswap(a.l[3]);
     q[1].w = b3_bswap(a.l[4]); q[1].z = b3_bswap(a.l[5]); q[1].y = b3_bswap(a.l[6]); q[1].x = b3_bswap(a.l[7]);
     q[0].w = b3_bswap(a.l[8]); q[0].z = b3_bswap(a.l[9]); q[0].y = b3_bswap(a.l[10]); q[0].x = b3_bswap(a.l[11]);

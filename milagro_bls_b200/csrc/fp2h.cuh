@@ -56,7 +56,7 @@ B3_FN_NOINLINE fp2h fp2h_mul_v(fp2h a, fp2h b) {
     fp ao, bo, nao, x1, x2;
     pair_xchg(ao, a.v);
     pair_xchg(bo, b.v);
-    fp_neg(nao, ao);
+    fp_neg_nr(nao, ao);
     const bool odd = pair_odd();
     fp_select(x1, odd, ao, a.v);          // even: a0      odd: a0
     fp_select(x2, odd, a.v, nao);         // even: -a1     odd: a1
@@ -70,7 +70,7 @@ B3_FN_NOINLINE fp2h fp2h_sqr_v(fp2h a) {
     pair_xchg(ao, a.v);
     const bool odd = pair_odd();
     fp_select(x, odd, ao, a.v);
-    fp_add(x, x, ao);                     // even: a0 + a1   odd: 2 a0
+    fp_add_nr(x, x, ao);                  // even: a0 + a1   odd: 2 a0     (< 4p: the first operand of the product)
     fp_sub(d, a.v, ao);
     fp_select(y, odd, a.v, d);            // even: a0 - a1   odd: a1
     fp2h r;

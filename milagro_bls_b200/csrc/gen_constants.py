@@ -170,6 +170,7 @@ def fp_arr(name, vs):
 out = ["// GENERATED by gen_constants.py -- do not edit.  Montgomery form, R = 2^384, little-endian u32 limbs.",
        "#pragma once", ""]
 out.append(fp_c("FP_P", p, raw=True))
+out.append(fp_c("FP_2P", 2 * p, raw=True))
 out.append(fp_c("FP_NIL", 0, raw=True))
 out.append(fp_c("FP_ONE", 1))
 out.append(fp_c("FP_RAW_ONE", 1, raw=True))

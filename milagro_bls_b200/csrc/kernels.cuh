@@ -144,7 +144,8 @@ __global__ void __launch_bounds__(B3_TPB) k_g1_decompress(const uint8_t* __restr
 // ---- device-resident public-key table (SURVEY.md 8(f)1; the reference pays PublicKey::from_bytes -- decompression + key_validate,
 // M/src/keys.rs:140-147 -- once per validator and then aggregates the decoded points, M/src/aggregates.rs:29-39) ----------------
 // Entry = (x, y) in Montgomery form, 96 bytes, read with six LDG.128 and used as is: no byte swap, no conversion, no checks per
-// use.  (0, 0) encodes infinity (it is not on the curve); x.l[11] = 0xffffffff (> p) marks an entry whose input was rejected.
+// use.  Coordinates are stored canonical.  (0, 0) encodes infinity (it is not on the curve); x.l[11] = 0xffffffff (> 2p) marks
+// an entry whose input was rejected.
 struct key_entry {
     fp x, y;
 };
@@ -171,7 +172,7 @@ __global__ void __launch_bounds__(B3_TPB) k_keytable_build(const uint8_t* __rest
     key_entry k;
     if (e) { k.x = FP_NIL; k.y = FP_NIL; k.x.l[11] = B3_KEY_INVALID; }
     else if (a.inf) { k.x = FP_NIL; k.y = FP_NIL; }
-    else { k.x = a.x; k.y = a.y; }
+    else { fp_canon(k.x, a.x); fp_canon(k.y, a.y); }
     out[i] = k;
     status[i] = e;
 }

@@ -41,7 +41,7 @@ B3_FN void fp2_one(fp2& r) { r.c0 = FP_ONE; r.c1 = FP_NIL; }
 B3_FN_NOINLINE fp2 fp2_mul_v(fp2 a, fp2 b) {
     fp2 r;
     fp na1;
-    fp_neg(na1, a.c1);
+    fp_neg_nr(na1, a.c1);
     fp_mul2_inl(r.c0, a.c0, b.c0, na1, b.c1);
     fp_mul2_inl(r.c1, a.c0, b.c1, a.c1, b.c0);
     return r;
@@ -51,7 +51,7 @@ B3_FN void fp2_mul(fp2& r, const fp2& a, const fp2& b) { r = fp2_mul_v(a, b); }
 B3_FN_NOINLINE fp2 fp2_sqr_v(fp2 a) {
     fp2 r;
     fp s, d, m;
-    fp_add(s, a.c0, a.c1);
+    fp_add_nr(s, a.c0, a.c1);             // < 4p: the first operand of the product
     fp_sub(d, a.c0, a.c1);
     fp_mul_inl(m, a.c0, a.c1);
     fp_mul_inl(r.c0, s, d);

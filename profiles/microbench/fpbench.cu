@@ -31,6 +31,7 @@ __global__ void __launch_bounds__(128) k_bench(uint32_t* out, int iters, uint32_
         if (V == 10) { fp2 a, b; a.c0 = x; a.c1 = z; b.c0 = y; b.c1 = w; a = fp2_mul_v(a, b); x = a.c0; z = a.c1; }
         if (V == 11) { fp2 a; a.c0 = x; a.c1 = z; a = fp2_sqr_v(a); x = a.c0; z = a.c1; }
         if (V == 12) { x = fp_sqr_v(x); }
+        if (V == 13) { g2h_jac P; P.x.v = x; P.y.v = y; P.z.v = z; pt_dbl(P, P); x = P.x.v; y = P.y.v; z = P.z.v; }
     }
     long long t1 = clock64();
     uint32_t r = 0;
@@ -82,5 +83,6 @@ int main() {
     run<10>("fp2_mul_v (1 thread)", N, 888);
     run<11>("fp2_sqr_v (1 thread)", N, 600);
     run<12>("fp_sqr_v (dedicated, 234 MACs)", N, 234);
+    run<13>("pt_dbl<fp2h> (lane pair)", N / 8, 0);
     return 0;
 }
