@@ -166,6 +166,19 @@ int b3_verify_multiple_indexed_dev(b3_ctx*, const b3_keytable*, const uint8_t* s
                                    const uint32_t* pk_off_dev, const uint8_t* msgs_dev, const uint32_t* msg_off_dev,
                                    const uint64_t* scalars_dev, size_t n, int* accept, int64_t* first_bad, uint8_t* gt576);
 
+/* Per-set verdicts for the most recent WHOLE verify_multiple call on this context (b3_verify_multiple, _checked, _indexed,
+ * _dev, _indexed_dev) that returned B3_OK.  n must be that call's n.  valid[j] = 1 iff set j ALONE passes
+ * verify_multiple_aggregate_signatures (M/src/aggregates.rs:261-316); n_invalid (nullable) = number of zeros.
+ * That is: sig_j passed subgroup_check_g2 and e(apk_j, H(msg_j)) == e(sig_j, G1); an aggregate key at infinity (an empty key
+ * range, or keys that cancel) contributes 1, so such a set is valid iff sig_j is infinity.  The verdict does not depend on
+ * the batch scalars and is computed without randomness.  Locate reuses what the batch call left on the device (hashes to
+ * G2 and their Miller lines, aggregate keys, parsed and checked signatures): the new work is one Miller point chain per
+ * signature and one two-pair Miller loop + final exponentiation per set.  If that call accepted, every valid[j] = 1 and
+ * nothing runs on the device.  Any other call on the context (including b3_sig_precheck, the _partial and sharded entries,
+ * b3_verify_batch, b3_hash_to_g2 and b3_keytable_append) ends the window: locate then returns B3_ERR_ARG, as it does for a
+ * wrong n.  Locate itself may be repeated and does not change the result of the next call. */
+int b3_verify_multiple_locate(b3_ctx*, size_t n, int32_t* valid, size_t* n_invalid);
+
 /* ---- batched verification of n INDEPENDENT items with one accept bit each (SURVEY.md 8(f)3: locating the bad set
  *      after a batch reject, or bulk verification of unrelated signatures).  Item i is, by `mode`,
  *        B3_ITEM_VERIFY          Signature::verify(sig_i, msg_i, pk_i)                           (M/src/signature.rs:27-40)

@@ -275,6 +275,36 @@ struct AggregateSignature {
         int accept = 0;
         return b3_verify_multiple_checked(c, apks.data(), nullptr, msgs.data(), off.data(), scalars.data(), n, &accept, nullptr) == B3_OK && accept == 1;
     }
+    // Extension (not in the reference): one verdict per set, true where the set ALONE passes
+    // verify_multiple_aggregate_signatures.  Exactly one scalar is drawn per set, in order, for every set (no stop at the first
+    // bad set: every set gets a verdict).  One b3_verify_multiple call; if it rejects, b3_verify_multiple_locate reads the
+    // per-set verdicts from what that call left on the device.  A malformed point or any other failure gives all false.
+    template <class Rng, class It>
+    static std::vector<bool> verify_multiple_aggregate_signatures_per_set(Rng& rng, It first, It last) {
+        std::vector<uint8_t> sigs, apks, msgs;
+        std::vector<uint32_t> off{0};
+        for (It it = first; it != last; ++it) {
+            const Set& s = *it;
+            sigs.insert(sigs.end(), s.signature->point.begin(), s.signature->point.end());
+            apks.insert(apks.end(), s.public_key->point.begin(), s.public_key->point.end());
+            msgs.insert(msgs.end(), s.msg, s.msg + s.msg_len);
+            off.push_back(static_cast<uint32_t>(msgs.size()));
+        }
+        const size_t n = off.size() - 1;
+        std::vector<uint64_t> scalars(n);
+        for (size_t j = 0; j < n; j++) scalars[j] = draw_scalar(rng);
+        std::vector<bool> out(n, false);
+        if (n == 0) return out;
+        b3_ctx* c = detail::ctx();
+        int accept = 0;
+        if (!c || b3_verify_multiple(c, sigs.data(), apks.data(), nullptr, msgs.data(), off.data(), scalars.data(), n, &accept, nullptr, nullptr) != B3_OK)
+            return out;
+        if (accept) return std::vector<bool>(n, true);
+        std::vector<int32_t> valid(n, 0);
+        if (b3_verify_multiple_locate(c, n, valid.data(), nullptr) != B3_OK) return out;
+        for (size_t j = 0; j < n; j++) out[j] = valid[j] != 0;
+        return out;
+    }
     // M/aggregates.rs:278-287: 8 bytes, i64::from_be_bytes(..).abs(), retry while 0 (i64::MIN, whose abs() overflows, is redrawn)
     template <class Rng>
     static uint64_t draw_scalar(Rng& rng) {

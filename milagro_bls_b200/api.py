@@ -313,6 +313,15 @@ class Engine:
                                                            ctypes.byref(ok), ctypes.byref(fb), gt.ctypes.data))
         return (bool(ok.value), int(fb.value), gt.tobytes()) if want_gt else (bool(ok.value), int(fb.value))
 
+    def verify_multiple_locate(self, n):
+        """Per-set verdicts of the preceding whole verify_multiple call on this engine (verify_multiple, _checked, _indexed,
+        _dev forms) that returned without raising: bool array, True where set j alone passes verify_multiple.  Any other call
+        in between, or a different n, raises RuntimeError (BadArgument)."""
+        valid = np.zeros(max(int(n), 1), dtype=np.int32)
+        n_bad = ctypes.c_size_t(0)
+        self._ck(self.L.b3_verify_multiple_locate(self.handle, int(n), valid.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), ctypes.byref(n_bad)))
+        return valid[:n].astype(bool)
+
     def sig_precheck(self, sigs192):
         """Phase one of the two-phase call: upload, parse and subgroup-check the signatures; returns first_bad (-1: all passed).
         The checked signatures stay in this context for verify_multiple_checked / verify_multiple_indexed(sigs192=None)."""
@@ -800,6 +809,26 @@ class AggregateSignature:
         accept = e.verify_multiple_checked(b"".join(k.point for _, k, _ in sets), None, b"".join(msgs), _offsets(msgs),
                                            np.array(scalars, dtype=np.uint64))
         return accept
+
+    @staticmethod
+    def verify_multiple_aggregate_signatures_per_set(rng, signature_sets, engine=None):
+        """Extension (the reference has no such function): one verdict per set, True where the set alone passes
+        verify_multiple_aggregate_signatures.  signature_sets as there.  Exactly one scalar is drawn per set, in order, for
+        every set -- there is no stop at the first bad set, since every set gets a verdict.  One batch call; if it rejects,
+        the sets are located from what it left on the device (Engine.verify_multiple_locate).  Malformed points raise
+        AmclError."""
+        e = engine or default_engine()
+        sets = list(signature_sets)
+        n = len(sets)
+        scalars = np.array([draw_scalar(rng) for _ in range(n)], dtype=np.uint64)
+        if n == 0:
+            return []
+        msgs = [bytes(m) for _, _, m in sets]
+        accept, _ = e.verify_multiple(b"".join(s.point for s, _, _ in sets), b"".join(k.point for _, k, _ in sets), None, b"".join(msgs),
+                                      _offsets(msgs), scalars)
+        if accept:
+            return [True] * n
+        return [bool(v) for v in e.verify_multiple_locate(n)]
 
     def __eq__(self, o):
         return isinstance(o, AggregateSignature) and self.point == o.point

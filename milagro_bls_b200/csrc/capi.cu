@@ -64,11 +64,14 @@ struct b3_ctx {
     dev_buf in_a, in_b, in_c, in_d, in_e, in_f;      // staged host inputs
     dev_buf g1j, g1j2, g1a, g2a_sig, g2j, g2j2, g2j_h, g2a, g2q, g1pp, qinf, f12a, f12b, lines, status, ok, misc, outb;
     dev_buf part;                   // this rank's packed partial (sharded calls)
+    dev_buf loc_lines, loc_qinf, loc_pp;   // b3_verify_multiple_locate only: signature lines, their qinf, unscaled keys in pairing form
     uint8_t* d_dst = nullptr;
     void* pin = nullptr;            // pinned host staging for the status read-back of a verify_multiple call
     size_t pin_cap = 0;
     long long h_init[2] = {0, 0};   // source of the small host-to-device initialisations (must outlive the async copy)
     size_t pre_n = (size_t)-1;      // number of signatures parsed + checked by b3_sig_precheck, (size_t)-1 = none
+    size_t loc_n = (size_t)-1;      // n of the whole verify_multiple call b3_verify_multiple_locate may read, (size_t)-1 = none
+    bool loc_accept = false;        // ... and whether that call accepted
 };
 
 #define CK(call)                                                                                   \
@@ -155,7 +158,7 @@ extern "C" void b3_ctx_destroy(b3_ctx* ctx) {
     for (int i = 0; i < 4; i++) if (ctx->aux[i]) cudaStreamSynchronize(ctx->aux[i]);
     dev_buf* bufs[] = {&ctx->in_a, &ctx->in_b, &ctx->in_c, &ctx->in_d, &ctx->in_e, &ctx->in_f, &ctx->g1j, &ctx->g1j2, &ctx->g1a,
                        &ctx->g2a_sig, &ctx->g2j, &ctx->g2j2, &ctx->g2j_h, &ctx->g2a, &ctx->g2q, &ctx->g1pp, &ctx->qinf, &ctx->lines, &ctx->f12a, &ctx->f12b, &ctx->status, &ctx->ok,
-                       &ctx->misc, &ctx->outb, &ctx->part};
+                       &ctx->misc, &ctx->outb, &ctx->part, &ctx->loc_lines, &ctx->loc_qinf, &ctx->loc_pp};
     if (ctx->pin) cudaFreeHost(ctx->pin);
     for (dev_buf* b : bufs) if (b->p) cudaFree(b->p);
     if (ctx->d_dst) cudaFree(ctx->d_dst);
@@ -257,6 +260,7 @@ static int begin(b3_ctx* ctx) {
     if (!ctx) return B3_ERR_ARG;
     CK(cudaSetDevice(ctx->device));
     ctx->wide_now = false;                    // set per call by the call_guard of the verify_multiple entries
+    ctx->loc_n = (size_t)-1;                  // any call may overwrite what b3_verify_multiple_locate reads (vm_whole re-enables it)
     return B3_OK;
 }
 
@@ -286,20 +290,20 @@ static int g2_sum(b3_ctx* ctx, g2_jac* a, g2_jac* b, size_t n, g2_jac** res, cud
     return B3_OK;
 }
 // Split multi-Miller loop (pairing.cuh), step 1: point chains of pairs [first, first + count) of an n_pairs product
-// -> lines in HBM (68 x n_pairs x 288 B).  May be issued on any stream as soon as those q's exist.
-static int miller_lines(b3_ctx* ctx, cudaStream_t strm, const g2_jac* q, size_t n_pairs, size_t first, size_t count) {
+// -> lines in HBM (68 x n_pairs x 288 B) and qinf (n_pairs x u32).  May be issued on any stream as soon as those q's exist.
+static int miller_lines(b3_ctx* ctx, cudaStream_t strm, const g2_jac* q, size_t n_pairs, size_t first, size_t count, dev_buf& lines, dev_buf& qinf) {
     if (count == 0) return B3_OK;
     int sp = span_begin(ctx, count <= 64 && first > 0 ? ST_MILLER_LINES_SUMS : ST_MILLER_LINES, strm);   // the few pairs of the signature MSM are timed apart
     if (ctx->wide_now || count <= 64)          // few pairs (the window sums of the signature MSM): always latency-bound
-        LAUNCH_ON(strm, k_miller_lines_q, nblk(4 * count), B3_TPB, q, n_pairs, first, count, (fp2*)ctx->lines.p, (uint32_t*)ctx->qinf.p);
+        LAUNCH_ON(strm, k_miller_lines_q, nblk(4 * count), B3_TPB, q, n_pairs, first, count, (fp2*)lines.p, (uint32_t*)qinf.p);
     else
-        LAUNCH_ON(strm, k_miller_lines, nblk(2 * count), B3_TPB, q, n_pairs, first, count, (fp2*)ctx->lines.p, (uint32_t*)ctx->qinf.p);
+        LAUNCH_ON(strm, k_miller_lines, nblk(2 * count), B3_TPB, q, n_pairs, first, count, (fp2*)lines.p, (uint32_t*)qinf.p);
     span_end(ctx, sp, strm);
     return B3_OK;
 }
-static int miller_reserve(b3_ctx* ctx, size_t n_pairs) {
-    CKR(ensure(ctx, ctx->lines, sizeof(fp2) * 3 * B3_MILLER_SLOTS * (n_pairs ? n_pairs : 1)));
-    CKR(ensure(ctx, ctx->qinf, 4 * (n_pairs ? n_pairs : 1)));
+static int miller_reserve(b3_ctx* ctx, size_t n_pairs, dev_buf& lines, dev_buf& qinf) {
+    CKR(ensure(ctx, lines, sizeof(fp2) * 3 * B3_MILLER_SLOTS * (n_pairs ? n_pairs : 1)));
+    CKR(ensure(ctx, qinf, 4 * (n_pairs ? n_pairs : 1)));
     return B3_OK;
 }
 // steps 2 and 3 (context stream): per-slot accumulation over all pairs, one cooperative closing chain -> *res
@@ -365,8 +369,8 @@ static int miller_finish(b3_ctx* ctx, const g1_pp* p, size_t n_pairs, fp12** res
 }
 // whole product on the context stream
 static int miller_product(b3_ctx* ctx, const g2_jac* q, const g1_pp* p, size_t n_pairs, fp12** res) {
-    CKR(miller_reserve(ctx, n_pairs));
-    CKR(miller_lines(ctx, ctx->stream, q, n_pairs, 0, n_pairs));
+    CKR(miller_reserve(ctx, n_pairs, ctx->lines, ctx->qinf));
+    CKR(miller_lines(ctx, ctx->stream, q, n_pairs, 0, n_pairs, ctx->lines, ctx->qinf));
     return miller_finish(ctx, p, n_pairs, res);
 }
 // final exponentiation of *m -> accept / gt on the host
@@ -728,6 +732,21 @@ extern "C" int b3_aggregate_verify(b3_ctx* ctx, const uint8_t sig192[192], const
 
 // ---- batched per-item verification (SURVEY.md 8(f)3): n independent items, one accept bit each ------------------------
 #define B3_ITEMS_PAIR_MIN 2048
+// Finishing kernel of n items on the context stream (k_items_finish*: pair 0 of item i = pair first0 + i of the np0-pair
+// table lines0, pair 1 = pair first1 + i of lines1).  CTA per item: ~1.5 ms per wave of 2 x 148 items; lane pair per item: one
+// item's latency (~12 ms) for any batch that fits the machine (17 ms at 16384 items, 33 ms at 32768) -- the crossover is near
+// 2.3 k items
+static void items_finish(b3_ctx* ctx, const fp2* lines0, const uint32_t* qinf0, size_t np0, size_t first0, const fp2* lines1, const uint32_t* qinf1,
+                         size_t np1, size_t first1, const g1_pp* keys, size_t n, const int32_t* st_sig, const int32_t* st_key, int key_rule,
+                         int32_t* accept, int32_t* status, uint8_t* gt) {
+    const bool per_pair = ctx->item_kernel == 3 || (ctx->item_kernel == 0 && n >= B3_ITEMS_PAIR_MIN);
+    if (per_pair)
+        LAUNCH(k_items_finish_p, (unsigned)((2 * n + B3_ITEMS_PAIR_TPB - 1) / B3_ITEMS_PAIR_TPB), B3_ITEMS_PAIR_TPB, lines0, qinf0, np0, first0,
+               lines1, qinf1, np1, first1, keys, n, st_sig, st_key, (const int32_t*)ctx->ok.p, key_rule, accept, status, gt);
+    else
+        LAUNCH(k_items_finish, (unsigned)n, B3_COOP_THREADS, lines0, qinf0, np0, first0, lines1, qinf1, np1, first1, keys, st_sig, st_key,
+               (const int32_t*)ctx->ok.p, key_rule, accept, status, gt);
+}
 static int verify_batch_core(b3_ctx* ctx, int mode, const uint8_t* d_sigs, const uint8_t* d_pks, const uint32_t* d_pk_off, size_t total_keys,
                              const uint8_t* d_msgs, const uint32_t* d_msg_off, size_t n, int32_t* d_accept, int32_t* d_status, uint8_t* d_gt) {
     CKR(ensure(ctx, ctx->g2a_sig, sizeof(g2_aff) * n));
@@ -736,7 +755,7 @@ static int verify_batch_core(b3_ctx* ctx, int mode, const uint8_t* d_sigs, const
     CKR(ensure(ctx, ctx->g1j, sizeof(g1_jac) * n));
     CKR(ensure(ctx, ctx->g1pp, sizeof(g1_pp) * n));
     CKR(ensure(ctx, ctx->g2q, sizeof(g2_jac) * 2 * n));
-    CKR(miller_reserve(ctx, 2 * n));
+    CKR(miller_reserve(ctx, 2 * n, ctx->lines, ctx->qinf));
     int32_t* d_st_sig = (int32_t*)ctx->status.p;
     int32_t* d_st_key = d_st_sig + n + 4;
     g2_jac* q = (g2_jac*)ctx->g2q.p;              // q[0 .. n) = signatures, q[n .. 2n) = H(msg)
@@ -753,7 +772,7 @@ static int verify_batch_core(b3_ctx* ctx, int mode, const uint8_t* d_sigs, const
     sp = span_begin(ctx, ST_HASH_TO_G2, s2);
     CKR(hash_to_g2_jac_dev(ctx, s2, d_msgs, d_msg_off, n, q + n));
     span_end(ctx, sp, s2);
-    CKR(miller_lines(ctx, s2, q, 2 * n, n, n));
+    CKR(miller_lines(ctx, s2, q, 2 * n, n, n, ctx->lines, ctx->qinf));
     // signatures: parse + on-curve, then the subgroup checks (aux0) beside their point chains (main)
     sp = span_begin(ctx, ST_COPY, sm);
     LAUNCH_ON(sm, k_g2_parse, nblk(n), B3_TPB, d_sigs, n, (g2_aff*)ctx->g2a_sig.p, d_st_sig, 1);
@@ -766,7 +785,7 @@ static int verify_batch_core(b3_ctx* ctx, int mode, const uint8_t* d_sigs, const
     sp = span_begin(ctx, ST_SIG_CHECK, s0);
     LAUNCH_ON(s0, k_g2_subgroup, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)d_st_sig, n, (int32_t*)ctx->ok.p);
     span_end(ctx, sp, s0);
-    CKR(miller_lines(ctx, sm, q, 2 * n, 0, n));
+    CKR(miller_lines(ctx, sm, q, 2 * n, 0, n, ctx->lines, ctx->qinf));
     // keys: aggregate (fast_aggregate_verify) or parse (verify / pre-aggregated) -> pairing form
     sp = span_begin(ctx, ST_AGGREGATE, s1);
     if (mode == B3_ITEM_FAST_AGGREGATE) {
@@ -785,16 +804,10 @@ static int verify_batch_core(b3_ctx* ctx, int mode, const uint8_t* d_sigs, const
     }
     CK(cudaEventRecord(ctx->ev[2], sm));
     sp = span_begin(ctx, ST_FINAL_EXP, sm);
-    // CTA per item: ~1.5 ms per wave of 2 x 148 items; lane pair per item: one item's latency (~12 ms) for any batch that fits
-    // the machine (17 ms at 16384 items, 33 ms at 32768) -- the crossover is near 2.3 k items
-    const bool per_pair = ctx->item_kernel == 3 || (ctx->item_kernel == 0 && n >= B3_ITEMS_PAIR_MIN);
-    if (per_pair)
-        LAUNCH_ON(sm, k_items_finish_p, (unsigned)((2 * n + B3_ITEMS_PAIR_TPB - 1) / B3_ITEMS_PAIR_TPB), B3_ITEMS_PAIR_TPB, (const fp2*)ctx->lines.p,
-                  (const uint32_t*)ctx->qinf.p, (const g1_pp*)keys, n, (const int32_t*)d_st_sig, (const int32_t*)d_st_key,
-                  (const int32_t*)ctx->ok.p, mode == B3_ITEM_VERIFY ? 0 : 1, d_accept, d_status, d_gt);
-    else
-        LAUNCH_ON(sm, k_items_finish, (unsigned)n, B3_COOP_THREADS, (const fp2*)ctx->lines.p, (const uint32_t*)ctx->qinf.p, (const g1_pp*)keys, n,
-                  (const int32_t*)d_st_sig, (const int32_t*)d_st_key, (const int32_t*)ctx->ok.p, mode == B3_ITEM_VERIFY ? 0 : 1, d_accept, d_status, d_gt);
+    const fp2* lines = (const fp2*)ctx->lines.p;
+    const uint32_t* qinf = (const uint32_t*)ctx->qinf.p;
+    items_finish(ctx, lines, qinf, 2 * n, 0, lines, qinf, 2 * n, n, keys, n, d_st_sig, d_st_key, mode == B3_ITEM_VERIFY ? B3_KEY_INF_PAIR : B3_KEY_INF_REJECT,
+                 d_accept, d_status, d_gt);
     span_end(ctx, sp, sm);
     CK(cudaEventRecord(ctx->ev[3], sm));
     return B3_OK;
@@ -986,6 +999,8 @@ struct vm_in {
     bool defer_sig = false;                 // run the subgroup checks beside the serial tail of the call instead of at its start (whole calls)
 };
 #define B3_FB_NONE 0x7fffffffffffffffLL
+// pairs of the batch product: H_j (j < n), then the signature sum S, or its 8 window sums from B3_MSM_MIN_SETS sets up
+static size_t vm_pairs(size_t n) { return n == 0 ? 0 : n + (n >= B3_MSM_MIN_SETS ? B3_MSM_WINDOWS : 1); }
 // one table entry per set (pre-aggregated keys held in the table)
 __global__ void __launch_bounds__(B3_TPB) k_g1_from_table(const key_entry* __restrict__ table, size_t n_table, const uint32_t* __restrict__ idx, size_t n,
                                                           g1_jac* out, int32_t* status) {
@@ -1028,7 +1043,7 @@ static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st
     sp = span_begin(ctx, ST_HASH_TO_G2, s2);
     CKR(hash_to_g2_jac_dev(ctx, s2, in.d_msgs, in.d_msg_off, n, q));
     span_end(ctx, sp, s2);
-    CKR(miller_lines(ctx, s2, q, n_total, 0, n));                 // the point chains need only H_j
+    CKR(miller_lines(ctx, s2, q, n_total, 0, n, ctx->lines, ctx->qinf));   // the point chains need only H_j
     // 1. signatures: parse + on-curve (main), subgroup check (M/src/aggregates.rs:274-276) on aux0 -- unless b3_sig_precheck
     //    already left the parsed signatures and their ok[] in the context
     if (!in.prechecked) {
@@ -1081,7 +1096,7 @@ static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st
         LAUNCH_ON(s3, k_set_neg_g1_pp, 1, 1, p + n);
     }
     span_end(ctx, sp, s3);
-    CKR(miller_lines(ctx, s3, q, n_total, n, n_total - n));       // ... and the window sums / S
+    CKR(miller_lines(ctx, s3, q, n_total, n, n_total - n, ctx->lines, ctx->qinf));   // ... and the window sums / S
     if (!ctx->serial) {
         cudaStream_t auxs[4] = {s0, s1, s2, s3};
         for (int k = 1; k < 4; k++) {
@@ -1142,7 +1157,7 @@ static int vm_enqueue(b3_ctx* ctx, const vm_in& in, fp12** res, long long** d_fi
         ctx->err = "b3_sig_precheck of the same signatures must precede a *_checked call on this context";
         return B3_ERR_ARG;
     }
-    const size_t n_total = n == 0 ? 0 : n + (n >= B3_MSM_MIN_SETS ? B3_MSM_WINDOWS : 1);
+    const size_t n_total = vm_pairs(n);
     // every buffer of the call is sized HERE, before the fork (ensure() may free / allocate, which synchronises the device)
     const size_t np = n >= B3_MSM_MIN_SETS ? msm_parts(msm_segs(n)) : 0;
     CKR(ensure(ctx, ctx->g2a_sig, sizeof(g2_aff) * (n + 1)));
@@ -1154,7 +1169,7 @@ static int vm_enqueue(b3_ctx* ctx, const vm_in& in, fp12** res, long long** d_fi
     CKR(ensure(ctx, ctx->g2j, sizeof(g2_jac) * (np > n + 1 ? np : n + 1)));
     CKR(ensure(ctx, ctx->g2j2, sizeof(g2_jac) * (n + 2 > (size_t)B3_MSM_WINDOWS * 256 ? n + 2 : (size_t)B3_MSM_WINDOWS * 256)));
     CKR(ensure(ctx, ctx->misc, 64));
-    CKR(miller_reserve(ctx, n_total));
+    CKR(miller_reserve(ctx, n_total, ctx->lines, ctx->qinf));
     CKR(miller_finish_reserve(ctx, n_total));
     if (ctx->pin_cap < 4 * (2 * n + 8) + 16) {
         if (ctx->pin) cudaFreeHost(ctx->pin);
@@ -1327,7 +1342,12 @@ static int vm_whole(b3_ctx* ctx, const vm_in& in0, int* accept, int64_t* first_b
     fp12* res;
     long long* d_fb;
     CKR(vm_enqueue(ctx, in, &res, &d_fb));
-    return vm_finish_whole(ctx, in.n, res, d_fb, accept, first_bad, gt576);
+    int ok = 0;
+    CKR(vm_finish_whole(ctx, in.n, res, d_fb, &ok, first_bad, gt576));
+    if (accept) *accept = ok;
+    ctx->loc_n = in.n;                         // the whole pipeline ran: its retained state serves b3_verify_multiple_locate
+    ctx->loc_accept = ok != 0;
+    return B3_OK;
 }
 static int vm_partial(b3_ctx* ctx, const vm_in& in, uint8_t* partial_dev) {
     call_guard guard(ctx, in.n);
@@ -1419,6 +1439,55 @@ extern "C" int b3_verify_multiple_indexed_dev(b3_ctx* ctx, const b3_keytable* tb
     vm_in in;
     CKR(vm_fill_dev(ctx, in, tbl, sigs192_dev, key_idx_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, 0));
     return vm_whole(ctx, in, accept, first_bad, gt576);
+}
+// Per-set verdicts of the preceding whole call: set j is valid iff sig_j passed subgroup_check_g2 and e(sig_j, -G1) e(H_j, apk_j)
+// == 1, which is verify_multiple over set j alone (c_j is invertible mod r, so the scalar drops out).  The call left in the
+// context everything but the signatures' point chains: H_j's lines (pairs [0, n) of `lines` at stride vm_pairs(n)), the
+// unscaled apk_j (g1j), the parsed signatures (g2a_sig), their subgroup results (ok) and the input statuses (status).  Only
+// the loc_* buffers, g2j and outb are written, so locate can be repeated and the next call starts from what it always does.
+// The stage times stay those of the batch call.
+extern "C" int b3_verify_multiple_locate(b3_ctx* ctx, size_t n, int32_t* valid, size_t* n_invalid) {
+    if (!ctx) return B3_ERR_ARG;
+    if (ctx->loc_n == (size_t)-1) {
+        ctx->err = "b3_verify_multiple_locate: the preceding call on this context is not a whole verify_multiple call that returned B3_OK";
+        return B3_ERR_ARG;
+    }
+    if (n != ctx->loc_n) {
+        ctx->err = "b3_verify_multiple_locate: n differs from the n of the preceding verify_multiple call";
+        return B3_ERR_ARG;
+    }
+    if (n && !valid) { ctx->err = "b3_verify_multiple_locate: valid is null"; return B3_ERR_ARG; }
+    if (n_invalid) *n_invalid = 0;
+    if (ctx->loc_accept) {                     // the batch accepted: so does every set
+        for (size_t j = 0; j < n; j++) valid[j] = 1;
+        return B3_OK;
+    }
+    CK(cudaSetDevice(ctx->device));
+    call_guard guard(ctx, n);
+    CKR(ensure(ctx, ctx->loc_pp, sizeof(g1_pp) * n));
+    CKR(miller_reserve(ctx, n, ctx->loc_lines, ctx->loc_qinf));
+    CKR(ensure(ctx, ctx->g2j, sizeof(g2_jac) * n));
+    CKR(ensure(ctx, ctx->outb, 4 * n));
+    int32_t* d_valid = (int32_t*)ctx->outb.p;
+    const int32_t* d_st_sig = (const int32_t*)ctx->status.p;
+    const int32_t* d_st_key = d_st_sig + n + 4;
+    CK(cudaEventRecord(ctx->ev[0], ctx->stream));
+    mark_reset(ctx);
+    LAUNCH(k_g2_aff_to_jac, nblk(n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, n, (g2_jac*)ctx->g2j.p);
+    CKR(miller_lines(ctx, ctx->stream, (const g2_jac*)ctx->g2j.p, n, 0, n, ctx->loc_lines, ctx->loc_qinf));
+    LAUNCH(k_g1_jac_to_pp, nblk(n), B3_TPB, (const g1_jac*)ctx->g1j.p, n, (g1_pp*)ctx->loc_pp.p);
+    CK(cudaEventRecord(ctx->ev[2], ctx->stream));
+    items_finish(ctx, (const fp2*)ctx->loc_lines.p, (const uint32_t*)ctx->loc_qinf.p, n, 0, (const fp2*)ctx->lines.p, (const uint32_t*)ctx->qinf.p,
+                 vm_pairs(n), 0, (const g1_pp*)ctx->loc_pp.p, n, d_st_sig, d_st_key, B3_KEY_BATCH, d_valid, nullptr, nullptr);
+    CK(cudaEventRecord(ctx->ev[3], ctx->stream));
+    CK(cudaEventRecord(ctx->ev[1], ctx->stream));
+    CKR(d2h(ctx, valid, d_valid, 4 * n));
+    CKR(sync(ctx));
+    cudaEventElapsedTime(&ctx->last_ms[0], ctx->ev[0], ctx->ev[1]);
+    if (cudaEventElapsedTime(&ctx->last_ms[1], ctx->ev[2], ctx->ev[3]) != cudaSuccess) ctx->last_ms[1] = 0.f;
+    cudaGetLastError();
+    if (n_invalid) for (size_t j = 0; j < n; j++) *n_invalid += valid[j] ? 0 : 1;
+    return B3_OK;
 }
 extern "C" int b3_verify_multiple_partial_dev(b3_ctx* ctx, const uint8_t* sigs192_dev, const uint8_t* pks96_dev, const uint32_t* pk_off_dev,
                                               const uint8_t* msgs_dev, const uint32_t* msg_off_dev, const uint64_t* scalars_dev, size_t n,

@@ -174,6 +174,8 @@ struct coop_item_pair {
     size_t idx;            // pair index in the line table
     fp ny, z3, xz;         // factors of the G1 member (g1_pp)
     int valid;             // 0: a member is infinity, the pair contributes 1
+    const fp2* lines;      // the pair's own line table of np pairs; null: the table passed to coop_item_miller
+    size_t np;
 };
 // thread tid < 6 scales Fp coordinate tid of the unscaled line (u0, l3, u5) by its factor of P -> coefficient w^0 / w^3 / w^5
 B3_FN void coop_line_load_p(fp12& line, const fp2* src, const coop_item_pair& pr, int tid) {
@@ -190,7 +192,8 @@ B3_FN void coop_set_p(fp12& r, bool one, int tid) {      // r = 0 or 1
     if (tid >= 12) return;
     reinterpret_cast<fp*>(&r)[tid] = (one && tid == 0) ? FP_ONE : FP_NIL;
 }
-// f = conj( prod_pairs f_{|x|,Q}(P) ); `line` is scratch.  lines[(slot * n_pairs + idx) * 3 ..] as written by k_miller_lines.
+// f = conj( prod_pairs f_{|x|,Q}(P) ); `line` is scratch.  lines[(slot * n_pairs + idx) * 3 ..] as written by k_miller_lines
+// (or the pair's own table, pr.lines / pr.np).
 COOP_FN void coop_item_miller(fp12& f, fp12& line, coop_ws& ws, const fp2* lines, size_t n_pairs, const coop_item_pair* pr, int npr) {
     const uint64_t x = B3_X_ABS;
     bool have = false;                                   // uniform over the CTA
@@ -203,7 +206,9 @@ COOP_FN void coop_item_miller(fp12& f, fp12& line, coop_ws& ws, const fp2* lines
             const size_t slot = s == 0 ? (size_t)it : (size_t)a;
             for (int q = 0; q < npr; q++) {
                 if (!pr[q].valid) continue;
-                COOP_PHASE(coop_line_load_p(line, lines + (slot * n_pairs + pr[q].idx) * 3, pr[q], tid));
+                const fp2* tab = pr[q].lines ? pr[q].lines : lines;
+                const size_t np = pr[q].lines ? pr[q].np : n_pairs;
+                COOP_PHASE(coop_line_load_p(line, tab + (slot * np + pr[q].idx) * 3, pr[q], tid));
                 if (have) coop_fp12_mul_line(f, f, line, ws);
                 else { coop_fp12_copy(f, line); have = true; }
             }

@@ -1114,36 +1114,51 @@ __global__ void __launch_bounds__(B3_COOP_THREADS) k_final_exp(const fp12* in, u
     if (tid == 0) *is_one = fp12_is_one(s.rr) ? 1 : 0;
 }
 
-// ---- batched PER-ITEM verification (b3_verify_batch): one CTA per item ------------------------------------------------
-// Item i owns pairs i = (sig_i, -G1) and n + i = (H(msg_i), key_i) of a 2n-pair line table.  The CTA folds the 2 x 68
-// lines into its own accumulator (sparse cooperative products), runs its own final exponentiation and writes the
-// item's accept bit, status and (optionally) GT bytes -- the shape of `ate2` + `fexp` (A/pair.rs:313-541) per item.
-// Items the reference rejects before any pairing (bad encoding, subgroup check, empty / infinite aggregate key;
-// M/src/signature.rs:29-31, M/src/aggregates.rs:179-198,229-236) skip the arithmetic altogether.
-__global__ void __launch_bounds__(B3_COOP_THREADS) k_items_finish(const fp2* __restrict__ lines, const uint32_t* __restrict__ qinf,
-                                                                  const g1_pp* __restrict__ keys, size_t n, const int32_t* st_sig,
-                                                                  const int32_t* st_key, const int32_t* sig_ok, int reject_inf_key,
+// ---- batched PER-ITEM verification (b3_verify_batch, b3_verify_multiple_locate): one CTA per item -------------------
+// Item i owns two pairs: (sig_i, -G1), whose lines are pair first0 + i of the np0-pair table lines0 (qinf0), and
+// (H(msg_i), key_i), pair first1 + i of the np1-pair table lines1 (b3_verify_batch passes its one 2n-pair table twice, with
+// first0 = 0 and first1 = n).  The CTA folds the 2 x 68 lines into its own accumulator (sparse cooperative products), runs
+// its own final exponentiation and writes the item's accept bit, status (nullable) and GT bytes (nullable) -- the shape of
+// `ate2` + `fexp` (A/pair.rs:313-541) per item.
+// Items the reference rejects before any pairing skip the arithmetic altogether, by key_rule:
+//   B3_KEY_INF_PAIR    bad encoding or subgroup check (M/src/signature.rs:29-31); an infinite key contributes 1
+//   B3_KEY_INF_REJECT  ... and an empty or infinite aggregate key (M/src/aggregates.rs:179-198,229-236)
+//   B3_KEY_BATCH       the rule of one set of verify_multiple (M/src/aggregates.rs:261-316): an empty key list
+//                      (B3_ERR_AGGREGATE_EMPTY_POINTS) or an infinite aggregate key rejects nothing, its pair contributes 1
+#define B3_KEY_INF_PAIR 0
+#define B3_KEY_INF_REJECT 1
+#define B3_KEY_BATCH 2
+__device__ __forceinline__ int item_code(const int32_t* st_sig, const int32_t* st_key, size_t i, int key_rule) {
+    const int kc = st_key[i];
+    return st_sig[i] ? st_sig[i] : (key_rule == B3_KEY_BATCH && kc == B3_ERR_AGGREGATE_EMPTY_POINTS_D) ? 0 : kc;
+}
+__global__ void __launch_bounds__(B3_COOP_THREADS) k_items_finish(const fp2* __restrict__ lines0, const uint32_t* __restrict__ qinf0, size_t np0,
+                                                                  size_t first0, const fp2* __restrict__ lines1, const uint32_t* __restrict__ qinf1,
+                                                                  size_t np1, size_t first1, const g1_pp* __restrict__ keys, const int32_t* st_sig,
+                                                                  const int32_t* st_key, const int32_t* sig_ok, int key_rule,
                                                                   int32_t* accept, int32_t* status, uint8_t* gt_wire) {
     __shared__ coop_fexp_ws s;
     __shared__ fp12 line;
     __shared__ coop_item_pair pr[2];
     const size_t i = blockIdx.x;
-    const int code = st_sig[i] ? st_sig[i] : st_key[i];
-    const bool rejected = code != 0 || !sig_ok[i] || (reject_inf_key && keys[i].inf);
+    const int code = item_code(st_sig, st_key, i, key_rule);
+    const bool rejected = code != 0 || !sig_ok[i] || (key_rule == B3_KEY_INF_REJECT && keys[i].inf);
     if (rejected) {                                    // uniform over the CTA
-        if (threadIdx.x == 0) { accept[i] = 0; status[i] = code; }
+        if (threadIdx.x == 0) { accept[i] = 0; if (status) status[i] = code; }
         if (gt_wire) for (int b = threadIdx.x; b < 576; b += blockDim.x) gt_wire[576 * i + b] = 0;
         return;
     }
     if (threadIdx.x == 0) {
-        pr[0].idx = i; pr[0].ny = G1_GEN_Y; pr[0].z3 = FP_ONE; pr[0].xz = G1_GEN_X;          // -G1: -(-y) = y
-        pr[0].valid = qinf[i] ? 0 : 1;
+        pr[0].idx = first0 + i; pr[0].ny = G1_GEN_Y; pr[0].z3 = FP_ONE; pr[0].xz = G1_GEN_X;          // -G1: -(-y) = y
+        pr[0].valid = qinf0[first0 + i] ? 0 : 1;
+        pr[0].lines = lines0; pr[0].np = np0;
         const g1_pp k = keys[i];
-        pr[1].idx = n + i; pr[1].ny = k.ny; pr[1].z3 = k.z3; pr[1].xz = k.xz;
-        pr[1].valid = (qinf[n + i] || k.inf) ? 0 : 1;
+        pr[1].idx = first1 + i; pr[1].ny = k.ny; pr[1].z3 = k.z3; pr[1].xz = k.xz;
+        pr[1].valid = (qinf1[first1 + i] || k.inf) ? 0 : 1;
+        pr[1].lines = lines1; pr[1].np = np1;
     }
     __syncthreads();
-    coop_item_miller(s.m, line, s.ws, lines, 2 * n, pr, 2);
+    coop_item_miller(s.m, line, s.ws, nullptr, 0, pr, 2);
     coop_final_exp(s);
     const int tid = (int)threadIdx.x;
     if (gt_wire && tid < 12) {                        // wire order w^0, w^3, w^1, w^4, w^2, w^5, each (re, im)
@@ -1153,7 +1168,7 @@ __global__ void __launch_bounds__(B3_COOP_THREADS) k_items_finish(const fp2* __r
         fp_from_mont(t, (tid & 1) ? c.c1 : c.c0);
         fp_raw_to_be(gt_wire + 576 * i + 48 * tid, t);
     }
-    if (tid == 0) { accept[i] = fp12_is_one(s.rr) ? 1 : 0; status[i] = 0; }
+    if (tid == 0) { accept[i] = fp12_is_one(s.rr) ? 1 : 0; if (status) status[i] = 0; }
 }
 
 // The same work with a LANE PAIR per item (large batches): a CTA per item keeps at most 2 x 148 items in flight, a lane pair per item
@@ -1171,26 +1186,27 @@ __device__ __noinline__ void item_fold_line_p(fp12_t<fp2h>& f, bool& have, const
     if (have) fp12_mul_by_line(f, l0, l3, l5);
     else { fp12_from_line(f, l0, l3, l5); have = true; }
 }
-__global__ void __launch_bounds__(B3_ITEMS_PAIR_TPB) k_items_finish_p(const fp2* __restrict__ lines, const uint32_t* __restrict__ qinf,
+__global__ void __launch_bounds__(B3_ITEMS_PAIR_TPB) k_items_finish_p(const fp2* __restrict__ lines0, const uint32_t* __restrict__ qinf0,
+                                                                       size_t np0, size_t first0, const fp2* __restrict__ lines1,
+                                                                       const uint32_t* __restrict__ qinf1, size_t np1, size_t first1,
                                                                        const g1_pp* __restrict__ keys, size_t n, const int32_t* st_sig,
-                                                                       const int32_t* st_key, const int32_t* sig_ok, int reject_inf_key,
+                                                                       const int32_t* st_key, const int32_t* sig_ok, int key_rule,
                                                                        int32_t* accept, int32_t* status, uint8_t* gt_wire) {
     const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
     if (i >= n) return;                                // both lanes of a pair leave together
     const bool odd = pair_odd();
-    const int code = st_sig[i] ? st_sig[i] : st_key[i];
+    const int code = item_code(st_sig, st_key, i, key_rule);
     const g1_pp key = keys[i];
-    if (code != 0 || !sig_ok[i] || (reject_inf_key && key.inf)) {
-        if (!odd) { accept[i] = 0; status[i] = code; }
+    if (code != 0 || !sig_ok[i] || (key_rule == B3_KEY_INF_REJECT && key.inf)) {
+        if (!odd) { accept[i] = 0; if (status) status[i] = code; }
         if (gt_wire) for (int b = odd ? 288 : 0; b < (odd ? 576 : 288); b++) gt_wire[576 * i + b] = 0;
         return;
     }
-    const bool valid0 = !qinf[i], valid1 = !(qinf[n + i] || key.inf);
+    const bool valid0 = !qinf0[first0 + i], valid1 = !(qinf1[first1 + i] || key.inf);
     const fp gy = G1_GEN_Y, one = FP_ONE, gx = G1_GEN_X;           // pair 0 = (sig_i, -G1): -(-y) = y
     fp12_t<fp2h> f, g;
     bool have = false;
     const uint64_t x = B3_X_ABS;
-    const size_t np = 2 * n;
     int a = B3_MILLER_DBL_SLOTS;
 #pragma unroll 1
     for (int it = 0; it < B3_MILLER_DBL_SLOTS; it++) {
@@ -1199,8 +1215,8 @@ __global__ void __launch_bounds__(B3_ITEMS_PAIR_TPB) k_items_finish_p(const fp2*
 #pragma unroll 1
         for (int s = 0; s < (add ? 2 : 1); s++) {
             const size_t slot = s == 0 ? (size_t)it : (size_t)a;
-            if (valid0) item_fold_line_p(f, have, lines + (slot * np + i) * 3, gy, one, gx);
-            if (valid1) item_fold_line_p(f, have, lines + (slot * np + n + i) * 3, key.ny, key.z3, key.xz);
+            if (valid0) item_fold_line_p(f, have, lines0 + (slot * np0 + first0 + i) * 3, gy, one, gx);
+            if (valid1) item_fold_line_p(f, have, lines1 + (slot * np1 + first1 + i) * 3, key.ny, key.z3, key.xz);
         }
         if (add) a++;
     }
@@ -1216,7 +1232,7 @@ __global__ void __launch_bounds__(B3_ITEMS_PAIR_TPB) k_items_finish_p(const fp2*
             fp_raw_to_be(gt_wire + 576 * i + 96 * k + (odd ? 48 : 0), t);
         }
     }
-    if (!odd) { accept[i] = is_one ? 1 : 0; status[i] = 0; }
+    if (!odd) { accept[i] = is_one ? 1 : 0; if (status) status[i] = 0; }
 }
 
 // ------------------------------------------------------------------------------------------------ roofline microbenchmarks

@@ -199,6 +199,50 @@ impl AggregateSignature {
         .unwrap_or(false)
     }
 
+    /// Extension (not in the reference): one verdict per set, `true` where the set ALONE passes
+    /// verify_multiple_aggregate_signatures -- what a caller needs after a batch returned false, to attribute and drop the bad
+    /// sets.  Exactly one scalar is drawn per set, in order, for every set (no stop at the first bad set: every set gets a
+    /// verdict).  One b3_verify_multiple call; if it rejects, b3_verify_multiple_locate reads the per-set verdicts from what
+    /// that call left on the device.  A malformed point (or any other failure) gives all `false`.
+    pub fn verify_multiple_aggregate_signatures_per_set<'a, R, I>(rng: &mut R, signature_sets: I) -> Vec<bool>
+    where
+        R: Rng + ?Sized,
+        I: Iterator<Item = (&'a AggregateSignature, &'a AggregatePublicKey, &'a [u8])>,
+    {
+        let (mut sigs, mut apks, mut msgs) = (Vec::new(), Vec::new(), Vec::new());
+        let mut off = vec![0u32];
+        for (s, k, m) in signature_sets {
+            sigs.extend_from_slice(&g2_wire(&s.point));
+            apks.extend_from_slice(&g1_wire(&k.point));
+            msgs.extend_from_slice(m);
+            off.push(msgs.len() as u32);
+        }
+        let n = off.len() - 1;
+        let scalars: Vec<u64> = (0..n).map(|_| draw_scalar(rng)).collect();
+        if n == 0 {
+            return Vec::new();
+        }
+        with_ctx(|ctx| {
+            let (mut accept, mut fb) = (0i32, -1i64);
+            let rc = unsafe {
+                b3_verify_multiple(ctx, sigs.as_ptr(), apks.as_ptr(), std::ptr::null(), msgs.as_ptr(), off.as_ptr(), scalars.as_ptr(), n,
+                                   &mut accept, &mut fb, std::ptr::null_mut())
+            };
+            if rc != B3_OK {
+                return vec![false; n];
+            }
+            if accept == 1 {
+                return vec![true; n];
+            }
+            let mut valid = vec![0i32; n];
+            if unsafe { b3_verify_multiple_locate(ctx, n, valid.as_mut_ptr(), std::ptr::null_mut()) } != B3_OK {
+                return vec![false; n];
+            }
+            valid.iter().map(|&v| v != 0).collect()
+        })
+        .unwrap_or_else(|| vec![false; n])
+    }
+
     /// aggregates.rs:319-322
     pub fn from_bytes(bytes: &[u8]) -> Result<AggregateSignature, AmclError> {
         Ok(AggregateSignature { point: Signature::from_bytes(bytes)?.point })
