@@ -8,6 +8,7 @@
 #include <dlfcn.h>
 #include <nccl.h>   // types only: the library is bound at run time (dlopen), see nccl()
 
+#include <algorithm>
 #include <condition_variable>
 #include <mutex>
 #include <string>
@@ -63,6 +64,7 @@ struct b3_ctx {
     // scratch (grown on demand, reused across calls)
     dev_buf in_a, in_b, in_c, in_d, in_e, in_f;      // staged host inputs
     dev_buf g1j, g1j2, g1a, g2a_sig, g2j, g2j2, g2j_h, g2a, g2q, g1pp, qinf, f12a, f12b, lines, status, ok, misc, outb;
+    dev_buf msm;                    // the signature MSM's digit sort: per-window index lists and bucket starts
     dev_buf part;                   // this rank's packed partial (sharded calls)
     dev_buf loc_lines, loc_qinf, loc_pp;   // b3_verify_multiple_locate only: signature lines, their qinf, unscaled keys in pairing form
     uint8_t* d_dst = nullptr;
@@ -158,7 +160,7 @@ extern "C" void b3_ctx_destroy(b3_ctx* ctx) {
     for (int i = 0; i < 4; i++) if (ctx->aux[i]) cudaStreamSynchronize(ctx->aux[i]);
     dev_buf* bufs[] = {&ctx->in_a, &ctx->in_b, &ctx->in_c, &ctx->in_d, &ctx->in_e, &ctx->in_f, &ctx->g1j, &ctx->g1j2, &ctx->g1a,
                        &ctx->g2a_sig, &ctx->g2j, &ctx->g2j2, &ctx->g2j_h, &ctx->g2a, &ctx->g2q, &ctx->g1pp, &ctx->qinf, &ctx->lines, &ctx->f12a, &ctx->f12b, &ctx->status, &ctx->ok,
-                       &ctx->misc, &ctx->outb, &ctx->part, &ctx->loc_lines, &ctx->loc_qinf, &ctx->loc_pp};
+                       &ctx->misc, &ctx->outb, &ctx->msm, &ctx->part, &ctx->loc_lines, &ctx->loc_qinf, &ctx->loc_pp};
     if (ctx->pin) cudaFreeHost(ctx->pin);
     for (dev_buf* b : bufs) if (b->p) cudaFree(b->p);
     if (ctx->d_dst) cudaFree(ctx->d_dst);
@@ -277,10 +279,12 @@ static int fp12_product(b3_ctx* ctx, fp12* a, fp12* b, size_t n, fp12** res) {
     *res = src;
     return B3_OK;
 }
-static int g2_sum(b3_ctx* ctx, g2_jac* a, g2_jac* b, size_t n, g2_jac** res, cudaStream_t strm = nullptr) {
+// sum of n G2 points in `a` (scratch `b`) by a pairwise tree, result left in *res; with keep > 1 the tree stops at `keep`
+// points, each the sum of n / keep consecutive inputs when n / keep is a power of two
+static int g2_sum(b3_ctx* ctx, g2_jac* a, g2_jac* b, size_t n, g2_jac** res, cudaStream_t strm = nullptr, size_t keep = 1) {
     g2_jac *src = a, *dst = b;
     if (!strm) strm = ctx->stream;
-    while (n > 1) {
+    while (n > keep) {
         size_t m = (n + 1) / 2;
         LAUNCH_ON(strm, k_g2_add_pairs, nblk(2 * m), B3_TPB, src, n, dst);
         g2_jac* t = src; src = dst; dst = t;
@@ -1081,15 +1085,17 @@ static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st
     // 5. S = sum_j [c_j] sig_j (M/src/aggregates.rs:303), on aux3: the context's own (highest-priority) stream is left to the
     //    end of the call
     sp = span_begin(ctx, ST_G2_MUL_SUM, s3);
+    g2_jac* s;
     if (n >= B3_MSM_MIN_SETS) {           // bucket method: 8 window sums, each its own pair against -[2^(8w)] G1
-        const unsigned segs = msm_segs(n);
-        const size_t np = msm_parts(segs);
-        LAUNCH_ON(s3, k_msm_bucket, nblk(2 * np), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, in.d_scalars, n, (g2_jac*)ctx->g2j.p, segs);
-        LAUNCH_ON(s3, k_msm_scale, nblk(2 * B3_MSM_WINDOWS * 256), B3_TPB, (const g2_jac*)ctx->g2j.p, (g2_jac*)ctx->g2j2.p, segs);
-        LAUNCH_ON(s3, k_msm_window_sum, B3_MSM_WINDOWS, 512, (g2_jac*)ctx->g2j2.p);
-        LAUNCH_ON(s3, k_msm_pairs, 1, 32, (const g2_jac*)ctx->g2j2.p, q + n, p + n);
+        const unsigned nr = msm_ranges(n);
+        uint32_t* idx = (uint32_t*)ctx->msm.p;
+        uint32_t* start = idx + B3_MSM_WINDOWS * n;
+        LAUNCH_ON(s3, k_msm_sort, B3_MSM_WINDOWS, 1024, in.d_scalars, n, idx, start);
+        LAUNCH_ON(s3, k_msm_walk, nblk(2 * (size_t)B3_MSM_WINDOWS * nr), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, idx, start, n, nr, msm_step(n),
+                  (g2_jac*)ctx->g2j.p);
+        CKR(g2_sum(ctx, (g2_jac*)ctx->g2j.p, (g2_jac*)ctx->g2j2.p, (size_t)B3_MSM_WINDOWS * nr, &s, s3, B3_MSM_WINDOWS));
+        LAUNCH_ON(s3, k_msm_pairs, 1, 32, s, q + n, p + n);
     } else {
-        g2_jac* s;
         LAUNCH_ON(s3, k_g2_mul_u64, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, in.d_scalars, n, (g2_jac*)ctx->g2j.p);
         CKR(g2_sum(ctx, (g2_jac*)ctx->g2j.p, (g2_jac*)ctx->g2j2.p, n, &s, s3));
         CK(cudaMemcpyAsync(q + n, s, sizeof(g2_jac), cudaMemcpyDeviceToDevice, s3));
@@ -1159,15 +1165,16 @@ static int vm_enqueue(b3_ctx* ctx, const vm_in& in, fp12** res, long long** d_fi
     }
     const size_t n_total = vm_pairs(n);
     // every buffer of the call is sized HERE, before the fork (ensure() may free / allocate, which synchronises the device)
-    const size_t np = n >= B3_MSM_MIN_SETS ? msm_parts(msm_segs(n)) : 0;
+    const size_t nr = n >= B3_MSM_MIN_SETS ? msm_ranges(n) : 0;     // ranges of the signature MSM per window
     CKR(ensure(ctx, ctx->g2a_sig, sizeof(g2_aff) * (n + 1)));
     CKR(ensure(ctx, ctx->status, 4 * (2 * n + 8)));
     CKR(ensure(ctx, ctx->ok, 4 * (n + 8)));
     CKR(ensure(ctx, ctx->g1j, sizeof(g1_jac) * (n + 1)));
     CKR(ensure(ctx, ctx->g1pp, sizeof(g1_pp) * (n + B3_MSM_WINDOWS)));
     CKR(ensure(ctx, ctx->g2q, sizeof(g2_jac) * (n + B3_MSM_WINDOWS)));
-    CKR(ensure(ctx, ctx->g2j, sizeof(g2_jac) * (np > n + 1 ? np : n + 1)));
-    CKR(ensure(ctx, ctx->g2j2, sizeof(g2_jac) * (n + 2 > (size_t)B3_MSM_WINDOWS * 256 ? n + 2 : (size_t)B3_MSM_WINDOWS * 256)));
+    CKR(ensure(ctx, ctx->g2j, sizeof(g2_jac) * std::max(n + 1, B3_MSM_WINDOWS * nr)));
+    CKR(ensure(ctx, ctx->g2j2, sizeof(g2_jac) * std::max(n + 2, B3_MSM_WINDOWS * nr / 2)));
+    if (nr) CKR(ensure(ctx, ctx->msm, 4 * (B3_MSM_WINDOWS * n + B3_MSM_WINDOWS * 257)));
     CKR(ensure(ctx, ctx->misc, 64));
     CKR(miller_reserve(ctx, n_total, ctx->lines, ctx->qinf));
     CKR(miller_finish_reserve(ctx, n_total));

@@ -523,109 +523,144 @@ __global__ void __launch_bounds__(B3_TPB) k_g2_mul_u256(const uint8_t* __restric
 }
 
 // ---- S = sum_j [c_j] sig_j as a multi-scalar multiplication (bucket method) -----------------------------------------
-// 64-bit scalars, B3_MSM_WINDOWS windows of 8 bits, 255 buckets per window.  ~15x fewer point operations than n
-// separate double-and-add ladders (M/src/aggregates.rs:303 does one g2mul per set).
-//   1. k_msm_bucket     : lane pair (w, b, seg) adds every signature of its scalar segment whose w-th digit equals b
-//   2. k_msm_scale      : lane pair (w, b) sums its segments and multiplies by b
-//   3. k_msm_window_sum : one CTA per window, W_w = sum_b [b] B_(w,b)
+// 64-bit scalars, B3_MSM_WINDOWS windows of 8 bits, buckets 1..255 per window (digit 0 adds nothing).
+//   1. k_msm_sort : per window, a stable counting sort of the set indices by digit -> idx[w][pos], bucket starts
+//   2. k_msm_walk : W_w = sum_b b B_b = sum_b R_b with R_b = sum_(b' >= b) B_b' (running sums), cut into ranges
+//   3. k_g2_add_pairs levels: the ranges of a window summed by a pairwise tree
 // and the windows are NOT recombined in G2 (56 dependent doublings): by bilinearity
 //   e(S, -G1) = prod_w e(W_w, -[2^(8w)] G1)
 // so the eight window sums become eight pairs of the multi-Miller loop against precomputed multiples of the
 // generator (G1_POW256_*).  The GT value is identical.
 #define B3_MSM_WINDOWS 8
 #define B3_MSM_BUCKETS 255
-#define B3_MSM_LIST 48
-// Segments per (window, bucket): the scalars are cut in `segs` contiguous ranges (2 * segs for the TOP window: the
-// reference's scalars are below 2^63, M/src/aggregates.rs:278-287, so its 127 non-empty buckets carry twice the load of
-// the others), one lane pair per (window, bucket, segment); segs grows with the batch so that a lane pair adds ~8 points.
-__host__ __device__ __forceinline__ unsigned msm_segs(size_t n) { return n <= 8192 ? 4u : 8u; }
-__host__ __device__ __forceinline__ size_t msm_parts(unsigned segs) { return (size_t)B3_MSM_BUCKETS * segs * (B3_MSM_WINDOWS + 1); }
-// (window, bucket index 0..254) -> first part and number of parts
-B3_FN size_t msm_part_base(unsigned w, unsigned bi, unsigned segs, unsigned& nseg) {
-    const bool top = w == B3_MSM_WINDOWS - 1;
-    nseg = top ? 2 * segs : segs;
-    return (size_t)w * B3_MSM_BUCKETS * segs + (size_t)bi * nseg;
-}
-__global__ void B3_LBH k_msm_bucket(const g2_aff* __restrict__ sigs, const uint64_t* __restrict__ k, size_t n, g2_jac* parts, unsigned segs) {
-    const size_t id = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
-    const bool live = id < msm_parts(segs);
-    const size_t blk = (size_t)B3_MSM_BUCKETS * segs;
-    unsigned w = (unsigned)(id / blk);
-    if (w > B3_MSM_WINDOWS - 1) w = B3_MSM_WINDOWS - 1;
-    const unsigned nseg = w == B3_MSM_WINDOWS - 1 ? 2 * segs : segs;
-    const size_t r = id - (size_t)w * blk;
-    const unsigned b = (unsigned)(r / nseg) + 1, seg = (unsigned)(r % nseg);
-    const size_t per = (n + nseg - 1) / nseg;
-    size_t j = seg * per, j1 = j + per;
-    if (j1 > n) j1 = n;
-    if (!live || j > n) j = j1 = 0;
-    g2h_jac acc;
-    pt_set_inf(acc);
-    // Scan first, add afterwards: the matching indices are collected in a list so that all lane pairs of a warp run
-    // their point additions together (adding inside the scan would serialise the warp: every pair matches at different
-    // positions).  The decisions to flush the lists and to stop are taken by the whole warp.
-    uint32_t list[B3_MSM_LIST];
-    int cnt = 0;
-    for (;;) {
-        if (j < j1) {
-            if ((unsigned)((k[j] >> (8 * w)) & 255u) == b) list[cnt++] = (uint32_t)j;
-            j++;
+// Target events per range of k_msm_walk (the actual length is 0.5x - 1x of this).  A range costs at most q point additions
+// whatever the digits: a signature event is one mixed addition (7M + 4S), and where STEPs follow each other (the empty
+// buckets around one full bucket when all scalars are equal) every STEP flushes the previous snapshot, one full addition
+// (11M + 5S) -- so a step-heavy range costs at most ~1.4x a signature-heavy one.
+#define B3_MSM_STEP 96
+// idx[w * n + pos]: the set indices ordered by the w-th digit, ties by index (a stable sort, so the order and with it every
+// value downstream is the same from run to run); start[w * 257 + d] = first position of digit d, start[w * 257 + 256] = n.
+// One CTA per window: a histogram, its scan, then 1024-set tiles ranked by __match_any_sync inside each warp and by a
+// column scan of the per-warp digit counts across the tile.
+__global__ void __launch_bounds__(1024) k_msm_sort(const uint64_t* __restrict__ k, size_t n, uint32_t* __restrict__ idx, uint32_t* __restrict__ start) {
+    __shared__ uint32_t run[256];
+    __shared__ uint32_t cnt[32][256];
+    const unsigned w = blockIdx.x, tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5, sh = 8 * w;
+    uint32_t* st = start + (size_t)w * 257;
+    uint32_t* out = idx + (size_t)w * n;
+    if (tid < 256) run[tid] = 0;
+    __syncthreads();
+    for (size_t j = tid; j < n; j += 1024) atomicAdd(&run[(unsigned)(k[j] >> sh) & 255u], 1u);
+    __syncthreads();
+    if (warp == 0) {                                 // exclusive scan of the 256 counts, 8 per lane
+        uint32_t c[8], s = 0;
+        for (int i = 0; i < 8; i++) { c[i] = run[lane * 8 + i]; s += c[i]; }
+        uint32_t x = s;
+        for (unsigned d = 1; d < 32; d <<= 1) {
+            const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
+            if (lane >= d) x += y;
         }
-        const bool more = __any_sync(0xffffffffu, j < j1);
-        if (!more || __any_sync(0xffffffffu, cnt == B3_MSM_LIST)) {
-            for (int t = 0; t < cnt; t++) {
-                g2h_aff p;
-                g2h_load(p, sigs[list[t]]);
-                pt_add_aff(acc, acc, p);
-            }
-            cnt = 0;
-        }
-        if (!more) break;
+        uint32_t base = x - s;
+        for (int i = 0; i < 8; i++) { run[lane * 8 + i] = base; st[lane * 8 + i] = base; base += c[i]; }
+        if (lane == 31) st[256] = base;
     }
-    if (live) g2h_store(parts[id], acc);
-}
-// out[w * 256 + (b - 1)] = [b] * sum_seg parts;  out[w * 256 + 255] = infinity (padding for the window tree)
-__global__ void B3_LBH k_msm_scale(const g2_jac* parts, g2_jac* out, unsigned segs) {
-    const size_t id = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
-    if (id >= (size_t)B3_MSM_WINDOWS * 256) return;
-    const unsigned w = (unsigned)(id >> 8), bi = (unsigned)(id & 255);
-    g2h_jac acc, t;
-    if (bi == B3_MSM_BUCKETS) {
-        pt_set_inf(t);
-    } else {
-        unsigned nseg;
-        const size_t base = msm_part_base(w, bi, segs, nseg);
-        g2h_load(acc, parts[base]);
-        for (unsigned sgm = 1; sgm < nseg; sgm++) {
-            g2h_load(t, parts[base + sgm]);
-            pt_add(acc, acc, t);
+    __syncthreads();
+    for (size_t t0 = 0; t0 < n; t0 += 1024) {
+        for (unsigned i = tid; i < 32 * 256; i += 1024) (&cnt[0][0])[i] = 0;
+        __syncthreads();
+        const size_t j = t0 + tid;
+        const bool live = j < n;
+        const unsigned d = live ? (unsigned)(k[j] >> sh) & 255u : 256u;
+        const unsigned peers = __match_any_sync(0xffffffffu, d);
+        const unsigned rank = __popc(peers & ((1u << lane) - 1u));
+        if (live && rank == 0) cnt[warp][d] = __popc(peers);
+        __syncthreads();
+        if (tid < 256) {                             // digit tid: where each warp's sets of this digit go
+            uint32_t s = run[tid];
+            for (int v = 0; v < 32; v++) { const uint32_t c = cnt[v][tid]; cnt[v][tid] = s; s += c; }
+            run[tid] = s;
         }
-        pt_mul_u64(t, acc, (uint64_t)(bi + 1));
-    }
-    g2h_store(out[id], t);
-}
-// one CTA (512 threads = 256 lane pairs) per window: in-place pairwise tree over vals[w * 256 .. w * 256 + 255];
-// the window sum is left in vals[w * 256]
-__global__ void __launch_bounds__(512) k_msm_window_sum(g2_jac* vals) {
-    g2_jac* v = vals + (size_t)blockIdx.x * 256;
-    const unsigned i = threadIdx.x >> 1;
-    for (unsigned s = 128; s >= 1; s >>= 1) {
-        if (i < s) {
-            g2h_jac a, b;
-            g2h_load(a, v[i]);
-            g2h_load(b, v[i + s]);
-            pt_add(a, a, b);
-            g2h_store(v[i], a);
-        }
-        __threadfence_block();
+        __syncthreads();
+        if (live) out[cnt[warp][d] + rank] = (uint32_t)j;
         __syncthreads();
     }
+}
+// Ranges of the running-sum walk.  A window's walk is a list of EVENTS, bucket b = 255 down to 1: the signatures of bucket b
+// (R += sig), then one STEP (T += R); at the end T = sum_b R_b = W_w.  The list has n - start[1] + 255 <= n + 255 events;
+// it is cut into msm_ranges(n) ranges (a power of two, so that the pairwise tree never pairs two windows) of msm_step(n)
+// events, one lane pair each: work per lane pair is bounded whatever the digits are (all sets in one bucket is the same
+// number of events as random scalars).
+__host__ __device__ __forceinline__ unsigned msm_ranges(size_t n) {
+    const size_t want = (n + B3_MSM_BUCKETS + B3_MSM_STEP - 1) / B3_MSM_STEP;
+    unsigned r = 1;
+    while (r < want) r <<= 1;
+    return r;
+}
+__host__ __device__ __forceinline__ unsigned msm_step(size_t n) { return (unsigned)((n + B3_MSM_BUCKETS + msm_ranges(n) - 1) / msm_ranges(n)); }
+// Lane pair (w, r) walks events [r q, r q + q) from zero with its own R and T.  The events before it hold the R_before of the
+// signatures already added, and each STEP of this range and after it would have added R_before too: out = T + [m] R + ...
+// with m = the number of STEPs from the range's end on (= the bucket the next event belongs to), summed over all ranges:
+// out[w * nr + r] = T_r + [m_r] R_r, and W_w = sum_r out[w * nr + r].
+// The signature additions run in lock step across the warp; a STEP only snapshots R, and the snapshots are added to T
+// warp-wide when some pair would need a second one (a branch taken by one pair costs the whole warp its full time).
+__global__ void B3_LBH k_msm_walk(const g2_aff* __restrict__ sigs, const uint32_t* __restrict__ idx, const uint32_t* __restrict__ start,
+                                  size_t n, unsigned nr, unsigned q, g2_jac* out) {
+    const size_t id = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+    const bool live = id < (size_t)B3_MSM_WINDOWS * nr;
+    const unsigned w = live ? (unsigned)(id / nr) : 0, r = (unsigned)(id % nr);
+    const uint32_t* st = start + (size_t)w * 257;
+    const uint32_t* ix = idx + (size_t)w * n;
+    const size_t total = n - st[1] + B3_MSM_BUCKETS;
+    size_t e = (size_t)r * q;
+    const size_t e1 = live && e < total ? (e + q < total ? e + q : total) : e;
+    // the event e: bucket b = the smallest b >= 1 whose block starts at or before e; blocks start at n - st[b + 1] + 255 - b
+    unsigned b = 0;
+    size_t pos = 0, end = 0;
+    if (e < e1) {
+        unsigned lo = 1, hi = B3_MSM_BUCKETS;
+        while (lo < hi) {
+            const unsigned mid = (lo + hi) >> 1;
+            if (n - st[mid + 1] + B3_MSM_BUCKETS - mid <= e) hi = mid; else lo = mid + 1;
+        }
+        b = lo;
+        end = st[b + 1];
+        pos = st[b] + (e - (n - end + B3_MSM_BUCKETS - b));
+    }
+    g2h_jac R, T, S;
+    pt_set_inf(R);
+    pt_set_inf(T);
+    bool pend = false;
+    for (unsigned t = 0; t < q; t++, e++) {
+        const bool ev = e < e1;
+        const bool step = ev && pos == end;
+        if (__any_sync(0xffffffffu, step && pend)) {
+            if (pend) pt_add(T, T, S);
+            pend = false;
+        }
+        if (step) {
+            S = R;
+            pend = true;
+            b--;
+            pos = st[b];
+            end = st[b + 1];
+        } else if (ev) {
+            g2h_aff p;
+            g2h_load(p, sigs[ix[pos]]);
+            pt_add_aff(R, R, p);
+            pos++;
+        }
+    }
+    if (pend) pt_add(T, T, S);
+    if (!live) return;
+    pt_mul_u64(R, R, (uint64_t)b);
+    pt_add(T, T, R);
+    g2h_store(out[id], T);
 }
 // pair members of the window sums: q[w] = W_w, p[w] = -[2^(8w)] G1 in pairing form
 __global__ void k_msm_pairs(const g2_jac* vals, g2_jac* q, g1_pp* p) {
     const unsigned w = threadIdx.x;
     if (w >= B3_MSM_WINDOWS) return;
-    q[w] = vals[(size_t)w * 256];
+    q[w] = vals[w];
     g1_pp a;
     a.xz = G1_POW256_X[w]; a.ny = G1_POW256_Y[w]; a.z3 = FP_ONE; a.inf = 0;
     p[w] = a;
