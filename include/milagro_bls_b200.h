@@ -166,8 +166,23 @@ int b3_verify_multiple_indexed_dev(b3_ctx*, const b3_keytable*, const uint8_t* s
                                    const uint32_t* pk_off_dev, const uint8_t* msgs_dev, const uint32_t* msg_off_dev,
                                    const uint64_t* scalars_dev, size_t n, int* accept, int64_t* first_bad, uint8_t* gt576);
 
+/* verify_multiple over sets that NAME THEIR MESSAGE BY INDEX (sync-committee messages, unaggregated attestations of one
+ * committee, aggregates of one slot): set j = (sigs192[j], the keys of set j as in b3_verify_multiple (table == NULL: 96-byte
+ * keys) or b3_verify_multiple_indexed (u32 indices into `table`), message msg_idx[j], scalars[j]); message k is
+ * msgs[msg_off[k] .. msg_off[k+1]), k < n_msgs.  Each distinct message is hashed once and gets one Miller pair, whose G1
+ * member is the sum of [c_j] apk_j over the sets naming it (prod_j e([c_j] apk_j, H) = e(sum_j [c_j] apk_j, H)); subgroup
+ * checks, key aggregation and the scalar multiplications stay per set.  accept, first_bad and gt576 equal, byte for byte,
+ * those of b3_verify_multiple / _indexed on the same sets with each set's message written out.  A message no set names, or
+ * whose sets' scaled keys sum to infinity, contributes 1.  sigs192 == NULL (host pointers only): the signatures of the
+ * preceding b3_sig_precheck.  device_pointers != 0: every input pointer is device memory.  n == 0 -> accept = 1; with n > 0,
+ * n_msgs == 0, any msg_idx[j] >= n_msgs or a zero scalar returns B3_ERR_ARG.  b3_verify_multiple_locate works after it. */
+int b3_verify_multiple_grouped(b3_ctx*, const b3_keytable* table, const uint8_t* sigs192, const void* keys,
+                               const uint32_t* pk_off, const uint8_t* msgs, const uint32_t* msg_off, size_t n_msgs,
+                               const uint32_t* msg_idx, const uint64_t* scalars, size_t n, int device_pointers, int* accept,
+                               int64_t* first_bad, uint8_t* gt576);
+
 /* Per-set verdicts for the most recent WHOLE verify_multiple call on this context (b3_verify_multiple, _checked, _indexed,
- * _dev, _indexed_dev) that returned B3_OK.  n must be that call's n.  valid[j] = 1 iff set j ALONE passes
+ * _dev, _indexed_dev, _grouped) that returned B3_OK.  n must be that call's n.  valid[j] = 1 iff set j ALONE passes
  * verify_multiple_aggregate_signatures (M/src/aggregates.rs:261-316); n_invalid (nullable) = number of zeros.
  * That is: sig_j passed subgroup_check_g2 and e(apk_j, H(msg_j)) == e(sig_j, G1); an aggregate key at infinity (an empty key
  * range, or keys that cancel) contributes 1, so such a set is valid iff sig_j is infinity.  The verdict does not depend on

@@ -19,6 +19,8 @@
 #include <array>
 #include <cstdint>
 #include <cstring>
+#include <map>
+#include <string>
 #include <utility>
 #include <vector>
 
@@ -274,6 +276,40 @@ struct AggregateSignature {
         if (first_bad >= 0) return false;
         int accept = 0;
         return b3_verify_multiple_checked(c, apks.data(), nullptr, msgs.data(), off.data(), scalars.data(), n, &accept, nullptr) == B3_OK && accept == 1;
+    }
+    // Extension (not in the reference): verify_multiple_aggregate_signatures with each DISTINCT message hashed and paired once
+    // (b3_verify_multiple_grouped), for batches whose sets repeat messages -- sync-committee messages, the unaggregated
+    // attestations of one committee.  Messages are deduplicated by their bytes.  The result and the RNG consumption are those
+    // of verify_multiple_aggregate_signatures: the same two phases, b3_sig_precheck -> draw -> the grouped call.
+    template <class Rng, class It>
+    static bool verify_multiple_aggregate_signatures_grouped(Rng& rng, It first, It last) {
+        std::vector<uint8_t> sigs, apks, msgs;
+        std::vector<uint32_t> off{0}, idx;
+        std::map<std::string, uint32_t> seen;
+        for (It it = first; it != last; ++it) {
+            const Set& s = *it;
+            sigs.insert(sigs.end(), s.signature->point.begin(), s.signature->point.end());
+            apks.insert(apks.end(), s.public_key->point.begin(), s.public_key->point.end());
+            const auto ins = seen.emplace(std::string(reinterpret_cast<const char*>(s.msg), s.msg_len), static_cast<uint32_t>(seen.size()));
+            if (ins.second) {
+                msgs.insert(msgs.end(), s.msg, s.msg + s.msg_len);
+                off.push_back(static_cast<uint32_t>(msgs.size()));
+            }
+            idx.push_back(ins.first->second);
+        }
+        const size_t n = idx.size();
+        if (n == 0) return true;
+        b3_ctx* c = detail::ctx();
+        if (!c) return false;
+        int64_t first_bad = -1;
+        if (b3_sig_precheck(c, sigs.data(), n, &first_bad) != B3_OK) return false;
+        const size_t n_draw = first_bad >= 0 ? static_cast<size_t>(first_bad) : n;
+        std::vector<uint64_t> scalars(n_draw);
+        for (size_t j = 0; j < n_draw; j++) scalars[j] = draw_scalar(rng);
+        if (first_bad >= 0) return false;
+        int accept = 0;
+        return b3_verify_multiple_grouped(c, nullptr, nullptr, apks.data(), nullptr, msgs.data(), off.data(), off.size() - 1, idx.data(),
+                                          scalars.data(), n, 0, &accept, nullptr, nullptr) == B3_OK && accept == 1;
     }
     // Extension (not in the reference): one verdict per set, true where the set ALONE passes
     // verify_multiple_aggregate_signatures.  Exactly one scalar is drawn per set, in order, for every set (no stop at the first

@@ -68,6 +68,7 @@ def lib():
         "b3_verify_multiple_dev": ([vp, vp, vp, vp, vp, vp, vp, sz, ip, i64p, u8p], ctypes.c_int),
         "b3_verify_multiple_indexed_dev": ([vp, vp, vp, vp, vp, vp, vp, vp, sz, ip, i64p, u8p], ctypes.c_int),
         "b3_verify_multiple_locate": ([vp, sz, i32p, ctypes.POINTER(sz)], ctypes.c_int),
+        "b3_verify_multiple_grouped": ([vp, vp, vp, vp, vp, vp, vp, sz, vp, vp, sz, ctypes.c_int, ip, i64p, u8p], ctypes.c_int),
         "b3_sig_precheck": ([vp, u8p, sz, i64p], ctypes.c_int),
         "b3_verify_multiple_checked": ([vp, u8p, vp, u8p, vp, vp, sz, ip, u8p], ctypes.c_int),
         "b3_keytable_create": ([vp, sz, ctypes.POINTER(vp)], ctypes.c_int),

@@ -313,6 +313,40 @@ class Engine:
                                                            ctypes.byref(ok), ctypes.byref(fb), gt.ctypes.data))
         return (bool(ok.value), int(fb.value), gt.tobytes()) if want_gt else (bool(ok.value), int(fb.value))
 
+    def verify_multiple_grouped(self, table, sigs192, keys, pk_offsets, msgs_blob, msg_offsets, msg_idx, scalars, want_gt=False):
+        """verify_multiple over sets that name their message by index: set j signs message msg_idx[j], message k is
+        msgs_blob[msg_offsets[k]:msg_offsets[k + 1]].  Each distinct message is hashed and paired once; the result equals
+        verify_multiple / verify_multiple_indexed on the expanded inputs.  table None: keys = 96-byte records, else u32 indices
+        into the KeyTable.  sigs192 None -> the signatures of the preceding sig_precheck.  Returns (accept, first_bad[, gt])."""
+        sc = np.ascontiguousarray(scalars, dtype=np.uint64)
+        n = len(sc)
+        mi = _u32(msg_idx)
+        moff = _u32(msg_offsets)
+        n_msgs = len(moff) - 1
+        _need(len(mi) == n, "verify_multiple_grouped: one message index per set")
+        _need(n_msgs >= 0 and moff[0] == 0 and int(moff[-1]) == len(msgs_blob),
+              "verify_multiple_grouped: message offsets must be n_msgs + 1 values ending at len(msgs)")
+        # the set-shaped checks of _vm_args on a one-message-per-set stand-in of the offsets
+        _, ps, pp, po, pm, _, sc, keep = self._vm_args(sigs192, keys, 96 if table is None else 4, pk_offsets, msgs_blob,
+                                                       np.array([0] * n + [len(msgs_blob)], dtype=np.uint32), sc, "verify_multiple_grouped")
+        ok = ctypes.c_int(0)
+        fb = ctypes.c_int64(-1)
+        gt = np.zeros(576, dtype=np.uint8)
+        self._ck(self.L.b3_verify_multiple_grouped(self.handle, None if table is None else table.handle, ps, pp, po, pm, moff.ctypes.data,
+                                                   max(n_msgs, 0), mi.ctypes.data, sc.ctypes.data, n, 0, ctypes.byref(ok), ctypes.byref(fb),
+                                                   gt.ctypes.data))
+        return (bool(ok.value), int(fb.value), gt.tobytes()) if want_gt else (bool(ok.value), int(fb.value))
+
+    def verify_multiple_grouped_dev(self, table, d_sigs, d_keys, d_pk_off, d_msgs, d_msg_off, n_msgs, d_msg_idx, d_scalars, n, want_gt=False):
+        """verify_multiple_grouped on inputs resident in HBM (device pointers as integers).  Returns (accept, first_bad[, gt])."""
+        ok = ctypes.c_int(0)
+        fb = ctypes.c_int64(-1)
+        gt = np.zeros(576, dtype=np.uint8)
+        self._ck(self.L.b3_verify_multiple_grouped(self.handle, None if table is None else table.handle, d_sigs, d_keys, d_pk_off, d_msgs,
+                                                   d_msg_off, int(n_msgs), d_msg_idx, d_scalars, int(n), 1, ctypes.byref(ok), ctypes.byref(fb),
+                                                   gt.ctypes.data))
+        return (bool(ok.value), int(fb.value), gt.tobytes()) if want_gt else (bool(ok.value), int(fb.value))
+
     def verify_multiple_locate(self, n):
         """Per-set verdicts of the preceding whole verify_multiple call on this engine (verify_multiple, _checked, _indexed,
         _dev forms) that returned without raising: bool array, True where set j alone passes verify_multiple.  Any other call
@@ -808,6 +842,32 @@ class AggregateSignature:
         msgs = [bytes(m) for _, _, m in sets]
         accept = e.verify_multiple_checked(b"".join(k.point for _, k, _ in sets), None, b"".join(msgs), _offsets(msgs),
                                            np.array(scalars, dtype=np.uint64))
+        return accept
+
+    @staticmethod
+    def verify_multiple_aggregate_signatures_grouped(rng, signature_sets, engine=None):
+        """Extension (the reference has no such function): verify_multiple_aggregate_signatures with every DISTINCT message
+        hashed and paired once (Engine.verify_multiple_grouped), for batches whose sets repeat messages.  Messages are
+        deduplicated by their bytes.  Result and RNG consumption are always those of verify_multiple_aggregate_signatures."""
+        e = engine or default_engine()
+        sets = list(signature_sets)
+        n = len(sets)
+        if n == 0:
+            return True
+        first_bad = e.sig_precheck(b"".join(s.point for s, _, _ in sets))
+        n_draw = first_bad if first_bad >= 0 else n
+        scalars = [draw_scalar(rng) for _ in range(n_draw)]
+        if first_bad >= 0:
+            return False
+        index, msgs, msg_idx = {}, [], []
+        for _, _, m in sets:
+            m = bytes(m)
+            if m not in index:
+                index[m] = len(msgs)
+                msgs.append(m)
+            msg_idx.append(index[m])
+        accept, _ = e.verify_multiple_grouped(None, None, b"".join(k.point for _, k, _ in sets), None, b"".join(msgs), _offsets(msgs),
+                                              np.array(msg_idx, dtype=np.uint32), np.array(scalars, dtype=np.uint64))
         return accept
 
     @staticmethod

@@ -67,6 +67,7 @@ struct b3_ctx {
     dev_buf msm;                    // the signature MSM's digit sort: per-window index lists and bucket starts
     dev_buf part;                   // this rank's packed partial (sharded calls)
     dev_buf loc_lines, loc_qinf, loc_pp;   // b3_verify_multiple_locate only: signature lines, their qinf, unscaled keys in pairing form
+    dev_buf in_g, grp;              // grouped calls: the sets' message indices; the sort by message and the group bounds
     uint8_t* d_dst = nullptr;
     void* pin = nullptr;            // pinned host staging for the status read-back of a verify_multiple call
     size_t pin_cap = 0;
@@ -74,6 +75,8 @@ struct b3_ctx {
     size_t pre_n = (size_t)-1;      // number of signatures parsed + checked by b3_sig_precheck, (size_t)-1 = none
     size_t loc_n = (size_t)-1;      // n of the whole verify_multiple call b3_verify_multiple_locate may read, (size_t)-1 = none
     bool loc_accept = false;        // ... and whether that call accepted
+    size_t loc_np = 0;              // ... the pair count of its line table (the stride of H's lines)
+    const uint32_t* loc_idx = nullptr;   // ... and for a grouped call the message index of every set (H's pair), else null
 };
 
 #define CK(call)                                                                                   \
@@ -160,7 +163,7 @@ extern "C" void b3_ctx_destroy(b3_ctx* ctx) {
     for (int i = 0; i < 4; i++) if (ctx->aux[i]) cudaStreamSynchronize(ctx->aux[i]);
     dev_buf* bufs[] = {&ctx->in_a, &ctx->in_b, &ctx->in_c, &ctx->in_d, &ctx->in_e, &ctx->in_f, &ctx->g1j, &ctx->g1j2, &ctx->g1a,
                        &ctx->g2a_sig, &ctx->g2j, &ctx->g2j2, &ctx->g2j_h, &ctx->g2a, &ctx->g2q, &ctx->g1pp, &ctx->qinf, &ctx->lines, &ctx->f12a, &ctx->f12b, &ctx->status, &ctx->ok,
-                       &ctx->misc, &ctx->outb, &ctx->msm, &ctx->part, &ctx->loc_lines, &ctx->loc_qinf, &ctx->loc_pp};
+                       &ctx->misc, &ctx->outb, &ctx->msm, &ctx->part, &ctx->loc_lines, &ctx->loc_qinf, &ctx->loc_pp, &ctx->in_g, &ctx->grp};
     if (ctx->pin) cudaFreeHost(ctx->pin);
     for (dev_buf* b : bufs) if (b->p) cudaFree(b->p);
     if (ctx->d_dst) cudaFree(ctx->d_dst);
@@ -737,18 +740,18 @@ extern "C" int b3_aggregate_verify(b3_ctx* ctx, const uint8_t sig192[192], const
 // ---- batched per-item verification (SURVEY.md 8(f)3): n independent items, one accept bit each ------------------------
 #define B3_ITEMS_PAIR_MIN 2048
 // Finishing kernel of n items on the context stream (k_items_finish*: pair 0 of item i = pair first0 + i of the np0-pair
-// table lines0, pair 1 = pair first1 + i of lines1).  CTA per item: ~1.5 ms per wave of 2 x 148 items; lane pair per item: one
-// item's latency (~12 ms) for any batch that fits the machine (17 ms at 16384 items, 33 ms at 32768) -- the crossover is near
-// 2.3 k items
+// table lines0, pair 1 = pair first1 + i of lines1, or pair idx1[i] when idx1 is not null).  CTA per item: ~1.5 ms per wave
+// of 2 x 148 items; lane pair per item: one item's latency (~12 ms) for any batch that fits the machine (17 ms at 16384 items,
+// 33 ms at 32768) -- the crossover is near 2.3 k items
 static void items_finish(b3_ctx* ctx, const fp2* lines0, const uint32_t* qinf0, size_t np0, size_t first0, const fp2* lines1, const uint32_t* qinf1,
-                         size_t np1, size_t first1, const g1_pp* keys, size_t n, const int32_t* st_sig, const int32_t* st_key, int key_rule,
+                         size_t np1, size_t first1, const uint32_t* idx1, const g1_pp* keys, size_t n, const int32_t* st_sig, const int32_t* st_key, int key_rule,
                          int32_t* accept, int32_t* status, uint8_t* gt) {
     const bool per_pair = ctx->item_kernel == 3 || (ctx->item_kernel == 0 && n >= B3_ITEMS_PAIR_MIN);
     if (per_pair)
         LAUNCH(k_items_finish_p, (unsigned)((2 * n + B3_ITEMS_PAIR_TPB - 1) / B3_ITEMS_PAIR_TPB), B3_ITEMS_PAIR_TPB, lines0, qinf0, np0, first0,
-               lines1, qinf1, np1, first1, keys, n, st_sig, st_key, (const int32_t*)ctx->ok.p, key_rule, accept, status, gt);
+               lines1, qinf1, np1, first1, idx1, keys, n, st_sig, st_key, (const int32_t*)ctx->ok.p, key_rule, accept, status, gt);
     else
-        LAUNCH(k_items_finish, (unsigned)n, B3_COOP_THREADS, lines0, qinf0, np0, first0, lines1, qinf1, np1, first1, keys, st_sig, st_key,
+        LAUNCH(k_items_finish, (unsigned)n, B3_COOP_THREADS, lines0, qinf0, np0, first0, lines1, qinf1, np1, first1, idx1, keys, st_sig, st_key,
                (const int32_t*)ctx->ok.p, key_rule, accept, status, gt);
 }
 static int verify_batch_core(b3_ctx* ctx, int mode, const uint8_t* d_sigs, const uint8_t* d_pks, const uint32_t* d_pk_off, size_t total_keys,
@@ -810,7 +813,7 @@ static int verify_batch_core(b3_ctx* ctx, int mode, const uint8_t* d_sigs, const
     sp = span_begin(ctx, ST_FINAL_EXP, sm);
     const fp2* lines = (const fp2*)ctx->lines.p;
     const uint32_t* qinf = (const uint32_t*)ctx->qinf.p;
-    items_finish(ctx, lines, qinf, 2 * n, 0, lines, qinf, 2 * n, n, keys, n, d_st_sig, d_st_key, mode == B3_ITEM_VERIFY ? B3_KEY_INF_PAIR : B3_KEY_INF_REJECT,
+    items_finish(ctx, lines, qinf, 2 * n, 0, lines, qinf, 2 * n, n, nullptr, keys, n, d_st_sig, d_st_key, mode == B3_ITEM_VERIFY ? B3_KEY_INF_PAIR : B3_KEY_INF_REJECT,
                  d_accept, d_status, d_gt);
     span_end(ctx, sp, sm);
     CK(cudaEventRecord(ctx->ev[3], sm));
@@ -996,6 +999,8 @@ struct vm_in {
     size_t total_keys = 0;
     const uint8_t* d_msgs = nullptr;
     const uint32_t* d_msg_off = nullptr;
+    size_t n_hash = 0;                      // messages hashed: n, or the n_msgs of a grouped call
+    const uint32_t* d_msg_idx = nullptr;    // grouped call: message of set j (n_hash messages); null: message j
     const uint64_t* d_scalars = nullptr;
     size_t n = 0;
     long long index_base = 0;
@@ -1003,8 +1008,9 @@ struct vm_in {
     bool defer_sig = false;                 // run the subgroup checks beside the serial tail of the call instead of at its start (whole calls)
 };
 #define B3_FB_NONE 0x7fffffffffffffffLL
-// pairs of the batch product: H_j (j < n), then the signature sum S, or its 8 window sums from B3_MSM_MIN_SETS sets up
-static size_t vm_pairs(size_t n) { return n == 0 ? 0 : n + (n >= B3_MSM_MIN_SETS ? B3_MSM_WINDOWS : 1); }
+// pairs of the batch product over n sets: the n_hash messages' H_k (k < n_hash), then the signature sum S, or its 8 window
+// sums from B3_MSM_MIN_SETS sets up
+static size_t vm_pairs(size_t n, size_t n_hash) { return n == 0 ? 0 : n_hash + (n >= B3_MSM_MIN_SETS ? B3_MSM_WINDOWS : 1); }
 // one table entry per set (pre-aggregated keys held in the table)
 __global__ void __launch_bounds__(B3_TPB) k_g1_from_table(const key_entry* __restrict__ table, size_t n_table, const uint32_t* __restrict__ idx, size_t n,
                                                           g1_jac* out, int32_t* status) {
@@ -1026,11 +1032,13 @@ __global__ void __launch_bounds__(B3_TPB) k_g1_from_table(const key_entry* __res
 // The forked region: the stages below are independent of each other; unless ctx->serial they run concurrently:
 //   main : parse signatures (... and, after the join, the end of the call: accumulation, closing chain)
 //   aux0 : subgroup checks of the parsed signatures               aux1 : aggregate keys -> P_j = [c_j] apk_j
-//   aux2 : H_j = hash_to_curve_g2(msg_j) -> their point chains    aux3 : S = sum_j [c_j] sig_j -> its point chains
+//   aux2 : H_k = hash_to_curve_g2(msg_k) -> their point chains    aux3 : S = sum_j [c_j] sig_j -> its point chains
+// (a grouped call hashes each of its n_hash messages once, and aux1 sums the P_j of the sets naming message k into pair k)
 // No allocation happens in here (every buffer is sized by the caller before the fork).
 static int vm_sig_checks(b3_ctx* ctx, const vm_in& in, const int32_t* d_st_sig, long long* d_first_bad);
-static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st_sig, int32_t* d_st_key, long long* d_first_bad, int32_t* d_zero) {
-    const size_t n = in.n;
+static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st_sig, int32_t* d_st_key, long long* d_first_bad, int32_t* d_zero,
+                     int32_t* d_range) {
+    const size_t n = in.n, nh = in.n_hash;
     g2_jac* q = (g2_jac*)ctx->g2q.p;
     g1_pp* p = (g1_pp*)ctx->g1pp.p;
     cudaStream_t sm = ctx->stream;
@@ -1045,9 +1053,9 @@ static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st
     // 4. H_j = hash_to_curve_g2(msg_j) (M/src/aggregates.rs:290) and its Miller point chain: the longest dependent chain of
     //    the batch, so it is issued FIRST (blocks are dispatched in launch order) on the high-priority stream
     sp = span_begin(ctx, ST_HASH_TO_G2, s2);
-    CKR(hash_to_g2_jac_dev(ctx, s2, in.d_msgs, in.d_msg_off, n, q));
+    CKR(hash_to_g2_jac_dev(ctx, s2, in.d_msgs, in.d_msg_off, nh, q));
     span_end(ctx, sp, s2);
-    CKR(miller_lines(ctx, s2, q, n_total, 0, n, ctx->lines, ctx->qinf));   // the point chains need only H_j
+    CKR(miller_lines(ctx, s2, q, n_total, 0, nh, ctx->lines, ctx->qinf));   // the point chains need only H_k
     // 1. signatures: parse + on-curve (main), subgroup check (M/src/aggregates.rs:274-276) on aux0 -- unless b3_sig_precheck
     //    already left the parsed signatures and their ok[] in the context
     if (!in.prechecked) {
@@ -1064,6 +1072,27 @@ static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st
     // partial record right after the closing chain, so its checks start here, with the call
     if (!in.defer_sig) CKR(vm_sig_checks(ctx, in, d_st_sig, d_first_bad));
     // 2. aggregate public keys; 3. P_j = [c_j] apk_j (M/src/aggregates.rs:293)
+    // grouped: the sets sorted by message first (it needs only msg_idx, so it runs while the keys are copied)
+    const uint32_t m = (uint32_t)nh;
+    uint32_t *perm = nullptr, *pos = nullptr, *lo = nullptr, *hi = nullptr;
+    if (in.d_msg_idx) {
+        uint32_t* w = (uint32_t*)ctx->grp.p;               // [perm0 | perm1 | pos] n each, then [lo | hi] m each
+        pos = w + 2 * n;
+        lo = w + 3 * n;
+        hi = lo + m;
+        int passes = 1;                                    // 8-bit digits of the largest index
+        while (passes < 4 && ((m - 1) >> (8 * passes)) != 0) passes++;
+        sp = span_begin(ctx, ST_G1_MUL, s1);
+        for (int t = 0; t < passes; t++) {
+            uint32_t* out = w + (size_t)(t & 1) * n;
+            LAUNCH_ON(s1, k_grp_sort, 1, 1024, in.d_msg_idx, n, m, 8u * t, t ? (const uint32_t*)perm : nullptr, out, t == passes - 1 ? pos : nullptr,
+                      t == 0 ? d_range : nullptr);
+            perm = out;
+        }
+        CK(cudaMemsetAsync(lo, 0, 8 * (size_t)m, s1));
+        LAUNCH_ON(s1, k_grp_bounds, nblk(n), B3_TPB, in.d_msg_idx, perm, n, m, lo, hi);
+        span_end(ctx, sp, s1);
+    }
     // host-pointer entries: the keys (96 % of the input bytes) or their indices are copied on THIS stream, so the transfer
     // overlaps hash_to_G2 and the signature work instead of preceding them
     if (in.h_pks) CK(cudaMemcpyAsync((void*)in.d_pks, in.h_pks, 96 * in.total_keys, cudaMemcpyHostToDevice, s1));
@@ -1079,8 +1108,18 @@ static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st
     }
     span_end(ctx, sp, s1);
     sp = span_begin(ctx, ST_G1_MUL, s1);
-    if (ctx->wide_now) LAUNCH_ON(s1, k_g1_mul_u64_pp_d, nblk(2 * n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, n, p, d_zero);
-    else LAUNCH_ON(s1, k_g1_mul_u64_pp, nblk(n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, n, p, d_zero);
+    if (in.d_msg_idx) {                   // [c_j] apk_j at the set's sorted position, a segmented tree per message, H_k's G1 member
+        g1_jac* a = (g1_jac*)ctx->g1j2.p;
+        if (ctx->wide_now) LAUNCH_ON(s1, k_g1_mul_u64_jac_d, nblk(2 * n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, pos, n, a, d_zero);
+        else LAUNCH_ON(s1, k_g1_mul_u64_jac, nblk(n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, pos, n, a, d_zero);
+        for (size_t step = 1; step < n; step <<= 1)
+            LAUNCH_ON(s1, k_grp_sum_level, nblk(n), B3_TPB, a, in.d_msg_idx, perm, lo, hi, n, m, step);
+        LAUNCH_ON(s1, k_grp_to_pp, nblk(m), B3_TPB, (const g1_jac*)a, lo, hi, m, p);
+    } else if (ctx->wide_now) {
+        LAUNCH_ON(s1, k_g1_mul_u64_pp_d, nblk(2 * n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, n, p, d_zero);
+    } else {
+        LAUNCH_ON(s1, k_g1_mul_u64_pp, nblk(n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, n, p, d_zero);
+    }
     span_end(ctx, sp, s1);
     // 5. S = sum_j [c_j] sig_j (M/src/aggregates.rs:303), on aux3: the context's own (highest-priority) stream is left to the
     //    end of the call
@@ -1094,15 +1133,15 @@ static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st
         LAUNCH_ON(s3, k_msm_walk, nblk(2 * (size_t)B3_MSM_WINDOWS * nr), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, idx, start, n, nr, msm_step(n),
                   (g2_jac*)ctx->g2j.p);
         CKR(g2_sum(ctx, (g2_jac*)ctx->g2j.p, (g2_jac*)ctx->g2j2.p, (size_t)B3_MSM_WINDOWS * nr, &s, s3, B3_MSM_WINDOWS));
-        LAUNCH_ON(s3, k_msm_pairs, 1, 32, s, q + n, p + n);
+        LAUNCH_ON(s3, k_msm_pairs, 1, 32, s, q + nh, p + nh);
     } else {
         LAUNCH_ON(s3, k_g2_mul_u64, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, in.d_scalars, n, (g2_jac*)ctx->g2j.p);
         CKR(g2_sum(ctx, (g2_jac*)ctx->g2j.p, (g2_jac*)ctx->g2j2.p, n, &s, s3));
-        CK(cudaMemcpyAsync(q + n, s, sizeof(g2_jac), cudaMemcpyDeviceToDevice, s3));
-        LAUNCH_ON(s3, k_set_neg_g1_pp, 1, 1, p + n);
+        CK(cudaMemcpyAsync(q + nh, s, sizeof(g2_jac), cudaMemcpyDeviceToDevice, s3));
+        LAUNCH_ON(s3, k_set_neg_g1_pp, 1, 1, p + nh);
     }
     span_end(ctx, sp, s3);
-    CKR(miller_lines(ctx, s3, q, n_total, n, n_total - n, ctx->lines, ctx->qinf));   // ... and the window sums / S
+    CKR(miller_lines(ctx, s3, q, n_total, nh, n_total - nh, ctx->lines, ctx->qinf));   // ... and the window sums / S
     if (!ctx->serial) {
         cudaStream_t auxs[4] = {s0, s1, s2, s3};
         for (int k = 1; k < 4; k++) {
@@ -1163,15 +1202,20 @@ static int vm_enqueue(b3_ctx* ctx, const vm_in& in, fp12** res, long long** d_fi
         ctx->err = "b3_sig_precheck of the same signatures must precede a *_checked call on this context";
         return B3_ERR_ARG;
     }
-    const size_t n_total = vm_pairs(n);
+    const size_t nh = in.n_hash;
+    const size_t n_total = vm_pairs(n, nh);
     // every buffer of the call is sized HERE, before the fork (ensure() may free / allocate, which synchronises the device)
     const size_t nr = n >= B3_MSM_MIN_SETS ? msm_ranges(n) : 0;     // ranges of the signature MSM per window
     CKR(ensure(ctx, ctx->g2a_sig, sizeof(g2_aff) * (n + 1)));
     CKR(ensure(ctx, ctx->status, 4 * (2 * n + 8)));
     CKR(ensure(ctx, ctx->ok, 4 * (n + 8)));
     CKR(ensure(ctx, ctx->g1j, sizeof(g1_jac) * (n + 1)));
-    CKR(ensure(ctx, ctx->g1pp, sizeof(g1_pp) * (n + B3_MSM_WINDOWS)));
-    CKR(ensure(ctx, ctx->g2q, sizeof(g2_jac) * (n + B3_MSM_WINDOWS)));
+    CKR(ensure(ctx, ctx->g1pp, sizeof(g1_pp) * (nh + B3_MSM_WINDOWS)));
+    CKR(ensure(ctx, ctx->g2q, sizeof(g2_jac) * (nh + B3_MSM_WINDOWS)));
+    if (in.d_msg_idx) {
+        CKR(ensure(ctx, ctx->g1j2, sizeof(g1_jac) * (n + 1)));
+        CKR(ensure(ctx, ctx->grp, 4 * (3 * n + 2 * nh)));
+    }
     CKR(ensure(ctx, ctx->g2j, sizeof(g2_jac) * std::max(n + 1, B3_MSM_WINDOWS * nr)));
     CKR(ensure(ctx, ctx->g2j2, sizeof(g2_jac) * std::max(n + 2, B3_MSM_WINDOWS * nr / 2)));
     if (nr) CKR(ensure(ctx, ctx->msm, 4 * (B3_MSM_WINDOWS * n + B3_MSM_WINDOWS * 257)));
@@ -1190,11 +1234,12 @@ static int vm_enqueue(b3_ctx* ctx, const vm_in& in, fp12** res, long long** d_fi
     int32_t* d_st_key = d_st_sig + n + 4;
     long long* d_first_bad = (long long*)ctx->misc.p;
     int32_t* d_zero = (int32_t*)((uint8_t*)ctx->misc.p + 8);
+    int32_t* d_range = d_zero + 1;                            // grouped: a message index >= n_hash
     ctx->h_init[0] = B3_FB_NONE;
     ctx->h_init[1] = 0;
     CK(cudaMemcpyAsync(d_first_bad, ctx->h_init, 16, cudaMemcpyHostToDevice, ctx->stream));
     if (n > 0) {
-        const int rc = vm_stages(ctx, in, n_total, d_st_sig, d_st_key, d_first_bad, d_zero);
+        const int rc = vm_stages(ctx, in, n_total, d_st_sig, d_st_key, d_first_bad, d_zero, d_range);
         if (rc != B3_OK) { vm_drain(ctx); return rc; }
     }
     // 6. Miller loops over the n + 8 (or n + 1) pairs: accumulation, then -- beside the subgroup checks -- the closing chain
@@ -1206,15 +1251,16 @@ static int vm_enqueue(b3_ctx* ctx, const vm_in& in, fp12** res, long long** d_fi
     CKR(miller_close(ctx, n_total));
     *d_first_bad_out = d_first_bad;
     if (n > 0) CK(cudaMemcpyAsync(ctx->pin, ctx->status.p, 4 * (2 * n + 8), cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaMemcpyAsync((uint8_t*)ctx->pin + 4 * (2 * n + 8), d_zero, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync((uint8_t*)ctx->pin + 4 * (2 * n + 8), d_zero, 8, cudaMemcpyDeviceToHost, ctx->stream));
     ctx->pre_n = (size_t)-1;                                  // a precheck is consumed by the call that follows it
     return B3_OK;
 }
 // after the stream synchronise: wire-format errors of the inputs (cannot happen for values that came out of the reference's
-// own types) and the zero-scalar flag
+// own types), the zero-scalar flag and the message-index flag of a grouped call
 static int vm_collect(b3_ctx* ctx, size_t n) {
     const int32_t* h = (const int32_t*)ctx->pin;
     if (h[2 * n + 8]) { ctx->err = "batch scalar 0: the draw rule of M/src/aggregates.rs:280-286 never yields it"; return B3_ERR_ARG; }
+    if (h[2 * n + 9]) { ctx->err = "msg_idx: a message index >= n_msgs"; return B3_ERR_ARG; }
     for (size_t i = 0; i < n; i++) {
         if (h[i]) return h[i];
         if (h[n + 4 + i] && h[n + 4 + i] != B3_ERR_AGGREGATE_EMPTY_POINTS) return h[n + 4 + i];
@@ -1288,11 +1334,13 @@ static int vm_finish_partial(b3_ctx* ctx, size_t n, fp12* res, long long* d_fb, 
 }
 // stages the HOST inputs of a call (signatures, offsets, messages, scalars now; keys / indices later, on the aggregation
 // stream) and fills `in`
+// (n_msgs messages: n, or the message count of a grouped call)
 static int vm_stage_host(b3_ctx* ctx, vm_in& in, const b3_keytable* tbl, const uint8_t* sigs192, const void* keys, const uint32_t* pk_off,
-                         const uint8_t* msgs, const uint32_t* msg_off, const uint64_t* scalars, size_t n, long long index_base) {
+                         const uint8_t* msgs, const uint32_t* msg_off, const uint64_t* scalars, size_t n, long long index_base, size_t n_msgs) {
     if (n && (!keys || !msg_off || !scalars)) return B3_ERR_ARG;
     CKR(scalars_nonzero(ctx, scalars, n));
     in.n = n;
+    in.n_hash = n_msgs;
     in.index_base = index_base;
     in.tbl = tbl;
     in.total_keys = pk_off ? pk_off[n] : n;
@@ -1301,8 +1349,8 @@ static int vm_stage_host(b3_ctx* ctx, vm_in& in, const b3_keytable* tbl, const u
     if (sigs192) CKR(h2d(ctx, ctx->in_a, sigs192, 192 * n));
     CKR(ensure(ctx, ctx->in_b, (tbl ? 4 : 96) * in.total_keys + 16));   // copied inside the call, on the aggregation stream
     if (pk_off) CKR(h2d(ctx, ctx->in_e, pk_off, 4 * (n + 1)));
-    CKR(h2d(ctx, ctx->in_c, msgs, msg_off[n]));
-    CKR(h2d(ctx, ctx->in_d, msg_off, 4 * (n + 1)));
+    CKR(h2d(ctx, ctx->in_c, msgs, msg_off[n_msgs]));
+    CKR(h2d(ctx, ctx->in_d, msg_off, 4 * (n_msgs + 1)));
     CKR(h2d(ctx, ctx->in_f, scalars, 8 * n));
     in.d_sigs = (const uint8_t*)ctx->in_a.p;
     if (tbl) { in.d_idx = (const uint32_t*)ctx->in_b.p; in.h_idx = (const uint32_t*)keys; }
@@ -1314,11 +1362,13 @@ static int vm_stage_host(b3_ctx* ctx, vm_in& in, const b3_keytable* tbl, const u
     return B3_OK;
 }
 static int vm_fill_dev(b3_ctx* ctx, vm_in& in, const b3_keytable* tbl, const uint8_t* sigs_dev, const void* keys_dev, const uint32_t* pk_off_dev,
-                       const uint8_t* msgs_dev, const uint32_t* msg_off_dev, const uint64_t* scalars_dev, size_t n, long long index_base) {
+                       const uint8_t* msgs_dev, const uint32_t* msg_off_dev, const uint64_t* scalars_dev, size_t n, long long index_base,
+                       size_t n_msgs) {
     if (n && (!sigs_dev || !keys_dev || !msg_off_dev || !scalars_dev)) return B3_ERR_ARG;
     CKR(dev_aligned(ctx, sigs_dev));
     if (!tbl) CKR(dev_aligned(ctx, keys_dev));
     in.n = n;
+    in.n_hash = n_msgs;
     in.index_base = index_base;
     in.tbl = tbl;
     in.d_sigs = sigs_dev;
@@ -1354,6 +1404,8 @@ static int vm_whole(b3_ctx* ctx, const vm_in& in0, int* accept, int64_t* first_b
     if (accept) *accept = ok;
     ctx->loc_n = in.n;                         // the whole pipeline ran: its retained state serves b3_verify_multiple_locate
     ctx->loc_accept = ok != 0;
+    ctx->loc_np = vm_pairs(in.n, in.n_hash);
+    ctx->loc_idx = in.d_msg_idx;
     return B3_OK;
 }
 static int vm_partial(b3_ctx* ctx, const vm_in& in, uint8_t* partial_dev) {
@@ -1371,7 +1423,7 @@ extern "C" int b3_verify_multiple(b3_ctx* ctx, const uint8_t* sigs192, const uin
     CKR(vm_begin(ctx));
     if (n && !sigs192) return B3_ERR_ARG;
     vm_in in;
-    CKR(vm_stage_host(ctx, in, nullptr, sigs192, pks96, pk_off, msgs, msg_off, scalars, n, 0));
+    CKR(vm_stage_host(ctx, in, nullptr, sigs192, pks96, pk_off, msgs, msg_off, scalars, n, 0, n));
     return vm_whole(ctx, in, accept, first_bad, gt576);
 }
 // The two-phase form that keeps the reference's RNG contract without doing anything twice (M/src/aggregates.rs:272-287: the
@@ -1408,7 +1460,7 @@ extern "C" int b3_verify_multiple_checked(b3_ctx* ctx, const uint8_t* pks96, con
     if (accept) *accept = 0;
     CKR(vm_begin(ctx));
     vm_in in;
-    CKR(vm_stage_host(ctx, in, nullptr, nullptr, pks96, pk_off, msgs, msg_off, scalars, n, 0));
+    CKR(vm_stage_host(ctx, in, nullptr, nullptr, pks96, pk_off, msgs, msg_off, scalars, n, 0, n));
     return vm_whole(ctx, in, accept, nullptr, gt576);
 }
 // verify_multiple over a key table: set j owns the table entries key_idx[pk_off[j] .. pk_off[j+1]) (pk_off == NULL: one entry per
@@ -1421,7 +1473,7 @@ extern "C" int b3_verify_multiple_indexed(b3_ctx* ctx, const b3_keytable* tbl, c
     CKR(vm_begin(ctx));
     if (!tbl) return B3_ERR_ARG;
     vm_in in;
-    CKR(vm_stage_host(ctx, in, tbl, sigs192, key_idx, pk_off, msgs, msg_off, scalars, n, 0));
+    CKR(vm_stage_host(ctx, in, tbl, sigs192, key_idx, pk_off, msgs, msg_off, scalars, n, 0, n));
     return vm_whole(ctx, in, accept, first_bad, gt576);
 }
 
@@ -1433,7 +1485,7 @@ extern "C" int b3_verify_multiple_dev(b3_ctx* ctx, const uint8_t* sigs192_dev, c
     if (first_bad) *first_bad = -1;
     CKR(vm_begin(ctx));
     vm_in in;
-    CKR(vm_fill_dev(ctx, in, nullptr, sigs192_dev, pks96_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, 0));
+    CKR(vm_fill_dev(ctx, in, nullptr, sigs192_dev, pks96_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, 0, n));
     return vm_whole(ctx, in, accept, first_bad, gt576);
 }
 extern "C" int b3_verify_multiple_indexed_dev(b3_ctx* ctx, const b3_keytable* tbl, const uint8_t* sigs192_dev, const uint32_t* key_idx_dev,
@@ -1444,12 +1496,42 @@ extern "C" int b3_verify_multiple_indexed_dev(b3_ctx* ctx, const b3_keytable* tb
     CKR(vm_begin(ctx));
     if (!tbl) return B3_ERR_ARG;
     vm_in in;
-    CKR(vm_fill_dev(ctx, in, tbl, sigs192_dev, key_idx_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, 0));
+    CKR(vm_fill_dev(ctx, in, tbl, sigs192_dev, key_idx_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, 0, n));
+    return vm_whole(ctx, in, accept, first_bad, gt576);
+}
+// verify_multiple with the message of set j named by msg_idx[j] among n_msgs messages: one hash_to_G2 and one Miller pair per
+// MESSAGE, whose G1 member is the sum of the scaled keys of the sets naming it (bilinearity).  The GT value is the one of the
+// ungrouped call on the expanded inputs.  keys = pks96 (tbl == NULL) or u32 indices into tbl; device_pointers != 0: every
+// input pointer is device memory (the range check of msg_idx is then a device flag read after the synchronise).
+extern "C" int b3_verify_multiple_grouped(b3_ctx* ctx, const b3_keytable* tbl, const uint8_t* sigs192, const void* keys, const uint32_t* pk_off,
+                                          const uint8_t* msgs, const uint32_t* msg_off, size_t n_msgs, const uint32_t* msg_idx,
+                                          const uint64_t* scalars, size_t n, int device_pointers, int* accept, int64_t* first_bad, uint8_t* gt576) {
+    if (accept) *accept = 0;
+    if (first_bad) *first_bad = -1;
+    CKR(vm_begin(ctx));
+    if (n && (!msg_idx || n_msgs == 0 || n_msgs > 0xffffffffu)) {
+        ctx->err = "b3_verify_multiple_grouped: n > 0 needs msg_idx and 0 < n_msgs < 2^32";
+        return B3_ERR_ARG;
+    }
+    const size_t nm = n ? n_msgs : 0;
+    vm_in in;
+    if (device_pointers) {
+        CKR(vm_fill_dev(ctx, in, tbl, sigs192, keys, pk_off, msgs, msg_off, scalars, n, 0, nm));
+        CKR(ensure(ctx, ctx->in_g, 4 * n + 4));
+        if (n) CK(cudaMemcpyAsync(ctx->in_g.p, msg_idx, 4 * n, cudaMemcpyDeviceToDevice, ctx->stream));   // locate reads it after the call
+    } else {
+        for (size_t j = 0; j < n; j++)
+            if (msg_idx[j] >= n_msgs) { ctx->err = "b3_verify_multiple_grouped: msg_idx[j] >= n_msgs"; return B3_ERR_ARG; }
+        CKR(vm_stage_host(ctx, in, tbl, sigs192, keys, pk_off, msgs, msg_off, scalars, n, 0, nm));
+        CKR(h2d(ctx, ctx->in_g, msg_idx, 4 * n));
+    }
+    if (n) in.d_msg_idx = (const uint32_t*)ctx->in_g.p;
     return vm_whole(ctx, in, accept, first_bad, gt576);
 }
 // Per-set verdicts of the preceding whole call: set j is valid iff sig_j passed subgroup_check_g2 and e(sig_j, -G1) e(H_j, apk_j)
 // == 1, which is verify_multiple over set j alone (c_j is invertible mod r, so the scalar drops out).  The call left in the
-// context everything but the signatures' point chains: H_j's lines (pairs [0, n) of `lines` at stride vm_pairs(n)), the
+// context everything but the signatures' point chains: H_j's lines (pairs [0, n) of `lines` at stride loc_np -- after a grouped
+// call pair msg_idx[j] of [0, n_msgs)), the
 // unscaled apk_j (g1j), the parsed signatures (g2a_sig), their subgroup results (ok) and the input statuses (status).  Only
 // the loc_* buffers, g2j and outb are written, so locate can be repeated and the next call starts from what it always does.
 // The stage times stay those of the batch call.
@@ -1485,7 +1567,7 @@ extern "C" int b3_verify_multiple_locate(b3_ctx* ctx, size_t n, int32_t* valid, 
     LAUNCH(k_g1_jac_to_pp, nblk(n), B3_TPB, (const g1_jac*)ctx->g1j.p, n, (g1_pp*)ctx->loc_pp.p);
     CK(cudaEventRecord(ctx->ev[2], ctx->stream));
     items_finish(ctx, (const fp2*)ctx->loc_lines.p, (const uint32_t*)ctx->loc_qinf.p, n, 0, (const fp2*)ctx->lines.p, (const uint32_t*)ctx->qinf.p,
-                 vm_pairs(n), 0, (const g1_pp*)ctx->loc_pp.p, n, d_st_sig, d_st_key, B3_KEY_BATCH, d_valid, nullptr, nullptr);
+                 ctx->loc_np, 0, ctx->loc_idx, (const g1_pp*)ctx->loc_pp.p, n, d_st_sig, d_st_key, B3_KEY_BATCH, d_valid, nullptr, nullptr);
     CK(cudaEventRecord(ctx->ev[3], ctx->stream));
     CK(cudaEventRecord(ctx->ev[1], ctx->stream));
     CKR(d2h(ctx, valid, d_valid, 4 * n));
@@ -1502,7 +1584,7 @@ extern "C" int b3_verify_multiple_partial_dev(b3_ctx* ctx, const uint8_t* sigs19
     CKR(vm_begin(ctx));
     if (!partial_dev) return B3_ERR_ARG;
     vm_in in;
-    CKR(vm_fill_dev(ctx, in, nullptr, sigs192_dev, pks96_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, index_base));
+    CKR(vm_fill_dev(ctx, in, nullptr, sigs192_dev, pks96_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, index_base, n));
     return vm_partial(ctx, in, partial_dev);
 }
 extern "C" int b3_verify_multiple_indexed_partial_dev(b3_ctx* ctx, const b3_keytable* tbl, const uint8_t* sigs192_dev, const uint32_t* key_idx_dev,
@@ -1511,7 +1593,7 @@ extern "C" int b3_verify_multiple_indexed_partial_dev(b3_ctx* ctx, const b3_keyt
     CKR(vm_begin(ctx));
     if (!partial_dev || !tbl) return B3_ERR_ARG;
     vm_in in;
-    CKR(vm_fill_dev(ctx, in, tbl, sigs192_dev, key_idx_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, index_base));
+    CKR(vm_fill_dev(ctx, in, tbl, sigs192_dev, key_idx_dev, pk_off_dev, msgs_dev, msg_off_dev, scalars_dev, n, index_base, n));
     return vm_partial(ctx, in, partial_dev);
 }
 // host-pointer form of the sharded call: this rank's shard comes from HOST memory (the keys are copied on the aggregation
@@ -1521,7 +1603,7 @@ extern "C" int b3_verify_multiple_partial(b3_ctx* ctx, const uint8_t* sigs192, c
     CKR(vm_begin(ctx));
     if (!partial_dev || (n && !sigs192)) return B3_ERR_ARG;
     vm_in in;
-    CKR(vm_stage_host(ctx, in, nullptr, sigs192, pks96, pk_off, msgs, msg_off, scalars, n, index_base));
+    CKR(vm_stage_host(ctx, in, nullptr, sigs192, pks96, pk_off, msgs, msg_off, scalars, n, index_base, n));
     return vm_partial(ctx, in, partial_dev);
 }
 extern "C" int b3_verify_multiple_indexed_partial(b3_ctx* ctx, const b3_keytable* tbl, const uint8_t* sigs192, const uint32_t* key_idx,
@@ -1530,7 +1612,7 @@ extern "C" int b3_verify_multiple_indexed_partial(b3_ctx* ctx, const b3_keytable
     CKR(vm_begin(ctx));
     if (!partial_dev || !tbl || (n && !sigs192)) return B3_ERR_ARG;
     vm_in in;
-    CKR(vm_stage_host(ctx, in, tbl, sigs192, key_idx, pk_off, msgs, msg_off, scalars, n, index_base));
+    CKR(vm_stage_host(ctx, in, tbl, sigs192, key_idx, pk_off, msgs, msg_off, scalars, n, index_base, n));
     return vm_partial(ctx, in, partial_dev);
 }
 // product of partials [i * stride], i < n_partials -> final exponentiation -> accept / first_bad / GT
@@ -1758,8 +1840,8 @@ extern "C" int b3_sharded_begin(b3_ctx* ctx, b3_comm* c, int lane, const b3_keyt
     CKR(vm_begin(ctx));
     if (!c || !ticket || (n && !sigs192)) return B3_ERR_ARG;
     vm_in in;
-    if (device_pointers) CKR(vm_fill_dev(ctx, in, tbl, sigs192, keys, pk_off, msgs, msg_off, scalars, n, index_base));
-    else CKR(vm_stage_host(ctx, in, tbl, sigs192, keys, pk_off, msgs, msg_off, scalars, n, index_base));
+    if (device_pointers) CKR(vm_fill_dev(ctx, in, tbl, sigs192, keys, pk_off, msgs, msg_off, scalars, n, index_base, n));
+    else CKR(vm_stage_host(ctx, in, tbl, sigs192, keys, pk_off, msgs, msg_off, scalars, n, index_base, n));
     CKR(ensure(ctx, ctx->part, B3_PARTIAL_BYTES));
     CKR(vm_partial(ctx, in, (uint8_t*)ctx->part.p));
     long long t = 0;

@@ -879,6 +879,135 @@ __global__ void __launch_bounds__(B3_TPB) k_g1_mul_u64_pp_d(const g1_jac* in, co
         out[i] = o;
     }
 }
+
+// ---- sets grouped by message (b3_verify_multiple_grouped) --------------------------------------------------------------
+// By bilinearity prod_(j in g) e([c_j] apk_j, H(m)) = e(sum_(j in g) [c_j] apk_j, H(m)): the sets naming message k share one
+// pair, whose G1 member is the sum of their scaled keys.  The set indices are sorted by message (k_grp_sort), each set's
+// [c_j] apk_j is written at its sorted position (k_g1_mul_u64_jac*), and every message's run of positions is reduced by a
+// segmented pairwise tree (k_grp_sum_level, one launch per level: log2(n) levels whatever the group sizes).
+// An out-of-range message index raises the flag and is read as message 0, so nothing indexes past the tables (the call is
+// then rejected).
+__device__ __forceinline__ uint32_t grp_key(const uint32_t* __restrict__ key, uint32_t j, uint32_t m) {
+    const uint32_t k = key[j];
+    return k < m ? k : 0u;
+}
+// One pass of an LSD radix sort of the set indices by message index: a stable counting sort by the 8-bit digit at `shift`
+// of the permutation `in` (nullptr: the identity) into `out`, one CTA, tiles ranked as in k_msm_sort.  pos (nullable, last
+// pass): pos[j] = sorted position of set j.  bad (nullable, first pass): set to 1 by any key >= m.
+__global__ void __launch_bounds__(1024) k_grp_sort(const uint32_t* __restrict__ key, size_t n, uint32_t m, unsigned shift,
+                                                   const uint32_t* __restrict__ in, uint32_t* __restrict__ out, uint32_t* __restrict__ pos,
+                                                   int32_t* bad) {
+    __shared__ uint32_t run[256];
+    __shared__ uint32_t cnt[32][256];
+    const unsigned tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
+    if (tid < 256) run[tid] = 0;
+    __syncthreads();
+    for (size_t j = tid; j < n; j += 1024) {
+        const uint32_t s = in ? in[j] : (uint32_t)j;
+        if (bad && key[s] >= m) *bad = 1;
+        atomicAdd(&run[(grp_key(key, s, m) >> shift) & 255u], 1u);
+    }
+    __syncthreads();
+    if (warp == 0) {                                 // exclusive scan of the 256 counts, 8 per lane
+        uint32_t c[8], s = 0;
+        for (int i = 0; i < 8; i++) { c[i] = run[lane * 8 + i]; s += c[i]; }
+        uint32_t x = s;
+        for (unsigned d = 1; d < 32; d <<= 1) {
+            const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
+            if (lane >= d) x += y;
+        }
+        uint32_t base = x - s;
+        for (int i = 0; i < 8; i++) { run[lane * 8 + i] = base; base += c[i]; }
+    }
+    __syncthreads();
+    for (size_t t0 = 0; t0 < n; t0 += 1024) {
+        for (unsigned i = tid; i < 32 * 256; i += 1024) (&cnt[0][0])[i] = 0;
+        __syncthreads();
+        const size_t j = t0 + tid;
+        const bool live = j < n;
+        const uint32_t s = live ? (in ? in[j] : (uint32_t)j) : 0u;
+        const unsigned d = live ? (grp_key(key, s, m) >> shift) & 255u : 256u;
+        const unsigned peers = __match_any_sync(0xffffffffu, d);
+        const unsigned rank = __popc(peers & ((1u << lane) - 1u));
+        if (live && rank == 0) cnt[warp][d] = __popc(peers);
+        __syncthreads();
+        if (tid < 256) {                             // digit tid: where each warp's sets of this digit go
+            uint32_t c0 = run[tid];
+            for (int v = 0; v < 32; v++) { const uint32_t c = cnt[v][tid]; cnt[v][tid] = c0; c0 += c; }
+            run[tid] = c0;
+        }
+        __syncthreads();
+        if (live) {
+            const uint32_t at = cnt[warp][d] + rank;
+            out[at] = s;
+            if (pos) pos[s] = at;
+        }
+        __syncthreads();
+    }
+}
+// [lo[k], hi[k]) = the sorted positions of the sets naming message k (both zeroed beforehand: an unnamed message keeps 0, 0)
+__global__ void __launch_bounds__(B3_TPB) k_grp_bounds(const uint32_t* __restrict__ key, const uint32_t* __restrict__ perm, size_t n, uint32_t m,
+                                                       uint32_t* lo, uint32_t* hi) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t k = grp_key(key, perm[i], m);
+    if (i == 0 || grp_key(key, perm[i - 1], m) != k) lo[k] = (uint32_t)i;
+    if (i + 1 == n || grp_key(key, perm[i + 1], m) != k) hi[k] = (uint32_t)(i + 1);
+}
+// P_j = [c_j] apk_j, Jacobian, at the sorted position pos[j]; zero_flag as in k_g1_mul_u64_pp
+__global__ void __launch_bounds__(B3_TPB) k_g1_mul_u64_jac(const g1_jac* in, const uint64_t* __restrict__ k, const uint32_t* __restrict__ pos, size_t n,
+                                                           g1_jac* out, int32_t* zero_flag) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    g1_jac p = in[i], r;
+    if (k[i] == 0) *zero_flag = 1;
+    pt_mul_u64_w4(r, p, k[i]);
+    out[pos[i]] = r;
+}
+// the same on LANE PAIRS (the latency mode, as k_g1_mul_u64_pp_d)
+__global__ void __launch_bounds__(B3_TPB) k_g1_mul_u64_jac_d(const g1_jac* in, const uint64_t* __restrict__ k, const uint32_t* __restrict__ pos, size_t n,
+                                                             g1_jac* out, int32_t* zero_flag) {
+    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+    if (i >= n) return;
+    g1d_jac p, r;
+    g1d_load(p, in[i]);
+    const uint64_t c = k[i];
+    if (c == 0) *zero_flag = 1;
+    pt_mul_u64_w4(r, p, c);
+    if (!pair_odd()) {
+        g1_jac o;
+        o.x = r.x.v; o.y = r.y.v; o.z = r.z.v;
+        out[pos[i]] = o;
+    }
+}
+// one level of the segmented tree: inside each message's run [lo, hi), position lo + r with r % (2 step) == 0 adds in position
+// lo + r + step.  After the levels step = 1, 2, 4, .. < n, position lo[k] holds the sum of the run (pt_add: complete, so
+// equal points -- one key and one scalar twice in a group -- and opposite points are exact).
+__global__ void __launch_bounds__(B3_TPB) k_grp_sum_level(g1_jac* a, const uint32_t* __restrict__ key, const uint32_t* __restrict__ perm,
+                                                          const uint32_t* __restrict__ lo, const uint32_t* __restrict__ hi, size_t n, uint32_t m,
+                                                          size_t step) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t k = grp_key(key, perm[i], m);
+    const size_t r = i - lo[k];
+    if ((r & (2 * step - 1)) != 0 || r + step >= hi[k] - lo[k]) return;
+    g1_jac x = a[i], y = a[i + step];
+    pt_add(x, x, y);
+    a[i] = x;
+}
+// group sums -> pairing form, message k = pair k (an unnamed message: infinity, its pair contributes 1)
+__global__ void __launch_bounds__(B3_TPB) k_grp_to_pp(const g1_jac* a, const uint32_t* __restrict__ lo, const uint32_t* __restrict__ hi, uint32_t m,
+                                                      g1_pp* out) {
+    const size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    g1_jac p;
+    if (hi[k] > lo[k]) p = a[lo[k]];
+    else pt_set_inf(p);
+    g1_pp r;
+    g1_pp_from_jac(r, p);
+    out[k] = r;
+}
+
 // constant pair member: -G1 generator
 __global__ void k_set_neg_g1_pp(g1_pp* out) {
     g1_pp a;
@@ -1151,8 +1280,9 @@ __global__ void __launch_bounds__(B3_COOP_THREADS) k_final_exp(const fp12* in, u
 
 // ---- batched PER-ITEM verification (b3_verify_batch, b3_verify_multiple_locate): one CTA per item -------------------
 // Item i owns two pairs: (sig_i, -G1), whose lines are pair first0 + i of the np0-pair table lines0 (qinf0), and
-// (H(msg_i), key_i), pair first1 + i of the np1-pair table lines1 (b3_verify_batch passes its one 2n-pair table twice, with
-// first0 = 0 and first1 = n).  The CTA folds the 2 x 68 lines into its own accumulator (sparse cooperative products), runs
+// (H(msg_i), key_i), pair first1 + i of the np1-pair table lines1 -- or pair idx1[i] when idx1 is not null (locate after a
+// grouped call: the message index of set i) -- (b3_verify_batch passes its one 2n-pair table twice, with first0 = 0 and
+// first1 = n).  The CTA folds the 2 x 68 lines into its own accumulator (sparse cooperative products), runs
 // its own final exponentiation and writes the item's accept bit, status (nullable) and GT bytes (nullable) -- the shape of
 // `ate2` + `fexp` (A/pair.rs:313-541) per item.
 // Items the reference rejects before any pairing skip the arithmetic altogether, by key_rule:
@@ -1169,7 +1299,8 @@ __device__ __forceinline__ int item_code(const int32_t* st_sig, const int32_t* s
 }
 __global__ void __launch_bounds__(B3_COOP_THREADS) k_items_finish(const fp2* __restrict__ lines0, const uint32_t* __restrict__ qinf0, size_t np0,
                                                                   size_t first0, const fp2* __restrict__ lines1, const uint32_t* __restrict__ qinf1,
-                                                                  size_t np1, size_t first1, const g1_pp* __restrict__ keys, const int32_t* st_sig,
+                                                                  size_t np1, size_t first1, const uint32_t* __restrict__ idx1,
+                                                                  const g1_pp* __restrict__ keys, const int32_t* st_sig,
                                                                   const int32_t* st_key, const int32_t* sig_ok, int key_rule,
                                                                   int32_t* accept, int32_t* status, uint8_t* gt_wire) {
     __shared__ coop_fexp_ws s;
@@ -1188,8 +1319,9 @@ __global__ void __launch_bounds__(B3_COOP_THREADS) k_items_finish(const fp2* __r
         pr[0].valid = qinf0[first0 + i] ? 0 : 1;
         pr[0].lines = lines0; pr[0].np = np0;
         const g1_pp k = keys[i];
-        pr[1].idx = first1 + i; pr[1].ny = k.ny; pr[1].z3 = k.z3; pr[1].xz = k.xz;
-        pr[1].valid = (qinf1[first1 + i] || k.inf) ? 0 : 1;
+        const size_t j1 = idx1 ? (size_t)idx1[i] : first1 + i;
+        pr[1].idx = j1; pr[1].ny = k.ny; pr[1].z3 = k.z3; pr[1].xz = k.xz;
+        pr[1].valid = (qinf1[j1] || k.inf) ? 0 : 1;
         pr[1].lines = lines1; pr[1].np = np1;
     }
     __syncthreads();
@@ -1224,7 +1356,8 @@ __device__ __noinline__ void item_fold_line_p(fp12_t<fp2h>& f, bool& have, const
 __global__ void __launch_bounds__(B3_ITEMS_PAIR_TPB) k_items_finish_p(const fp2* __restrict__ lines0, const uint32_t* __restrict__ qinf0,
                                                                        size_t np0, size_t first0, const fp2* __restrict__ lines1,
                                                                        const uint32_t* __restrict__ qinf1, size_t np1, size_t first1,
-                                                                       const g1_pp* __restrict__ keys, size_t n, const int32_t* st_sig,
+                                                                       const uint32_t* __restrict__ idx1, const g1_pp* __restrict__ keys, size_t n,
+                                                                       const int32_t* st_sig,
                                                                        const int32_t* st_key, const int32_t* sig_ok, int key_rule,
                                                                        int32_t* accept, int32_t* status, uint8_t* gt_wire) {
     const size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
@@ -1237,7 +1370,8 @@ __global__ void __launch_bounds__(B3_ITEMS_PAIR_TPB) k_items_finish_p(const fp2*
         if (gt_wire) for (int b = odd ? 288 : 0; b < (odd ? 576 : 288); b++) gt_wire[576 * i + b] = 0;
         return;
     }
-    const bool valid0 = !qinf0[first0 + i], valid1 = !(qinf1[first1 + i] || key.inf);
+    const size_t j1 = idx1 ? (size_t)idx1[i] : first1 + i;
+    const bool valid0 = !qinf0[first0 + i], valid1 = !(qinf1[j1] || key.inf);
     const fp gy = G1_GEN_Y, one = FP_ONE, gx = G1_GEN_X;           // pair 0 = (sig_i, -G1): -(-y) = y
     fp12_t<fp2h> f, g;
     bool have = false;
@@ -1251,7 +1385,7 @@ __global__ void __launch_bounds__(B3_ITEMS_PAIR_TPB) k_items_finish_p(const fp2*
         for (int s = 0; s < (add ? 2 : 1); s++) {
             const size_t slot = s == 0 ? (size_t)it : (size_t)a;
             if (valid0) item_fold_line_p(f, have, lines0 + (slot * np0 + first0 + i) * 3, gy, one, gx);
-            if (valid1) item_fold_line_p(f, have, lines1 + (slot * np1 + first1 + i) * 3, key.ny, key.z3, key.xz);
+            if (valid1) item_fold_line_p(f, have, lines1 + (slot * np1 + j1) * 3, key.ny, key.z3, key.xz);
         }
         if (add) a++;
     }

@@ -199,6 +199,54 @@ impl AggregateSignature {
         .unwrap_or(false)
     }
 
+    /// Extension (not in the reference): verify_multiple_aggregate_signatures with every DISTINCT message hashed and paired
+    /// once (b3_verify_multiple_grouped), for batches whose sets repeat messages -- sync-committee messages, the unaggregated
+    /// attestations of one committee.  Messages are deduplicated by their bytes.  The result and the RNG consumption are those
+    /// of verify_multiple_aggregate_signatures: b3_sig_precheck -> draw -> the grouped call.
+    pub fn verify_multiple_aggregate_signatures_grouped<'a, R, I>(rng: &mut R, signature_sets: I) -> bool
+    where
+        R: Rng + ?Sized,
+        I: Iterator<Item = (&'a AggregateSignature, &'a AggregatePublicKey, &'a [u8])>,
+    {
+        let (mut sigs, mut apks, mut msgs) = (Vec::new(), Vec::new(), Vec::new());
+        let (mut off, mut idx) = (vec![0u32], Vec::new());
+        let mut seen: std::collections::HashMap<&'a [u8], u32> = std::collections::HashMap::new();
+        for (s, k, m) in signature_sets {
+            sigs.extend_from_slice(&g2_wire(&s.point));
+            apks.extend_from_slice(&g1_wire(&k.point));
+            let next = seen.len() as u32;
+            let id = *seen.entry(m).or_insert_with(|| {
+                msgs.extend_from_slice(m);
+                off.push(msgs.len() as u32);
+                next
+            });
+            idx.push(id);
+        }
+        let n = idx.len();
+        if n == 0 {
+            return true;
+        }
+        with_ctx(|ctx| {
+            let mut first_bad = -1i64;
+            if unsafe { b3_sig_precheck(ctx, sigs.as_ptr(), n, &mut first_bad) } != B3_OK {
+                return false;
+            }
+            let n_draw = if first_bad >= 0 { first_bad as usize } else { n };
+            let scalars: Vec<u64> = (0..n_draw).map(|_| draw_scalar(rng)).collect();
+            if first_bad >= 0 {
+                return false;
+            }
+            let (mut accept, mut fb) = (0i32, -1i64);
+            let rc = unsafe {
+                b3_verify_multiple_grouped(ctx, std::ptr::null(), std::ptr::null(), apks.as_ptr() as *const std::os::raw::c_void,
+                                           std::ptr::null(), msgs.as_ptr(), off.as_ptr(), off.len() - 1, idx.as_ptr(), scalars.as_ptr(), n, 0,
+                                           &mut accept, &mut fb, std::ptr::null_mut())
+            };
+            rc == B3_OK && accept == 1
+        })
+        .unwrap_or(false)
+    }
+
     /// Extension (not in the reference): one verdict per set, `true` where the set ALONE passes
     /// verify_multiple_aggregate_signatures -- what a caller needs after a batch returned false, to attribute and drop the bad
     /// sets.  Exactly one scalar is drawn per set, in order, for every set (no stop at the first bad set: every set gets a

@@ -70,6 +70,10 @@ extern "C" {
     pub fn b3_verify_multiple_indexed_dev(ctx: *mut b3_ctx, t: *const b3_keytable, sigs192_dev: *const u8, key_idx_dev: *const u32,
                                           pk_off_dev: *const u32, msgs_dev: *const u8, msg_off_dev: *const u32, scalars_dev: *const u64,
                                           n: usize, accept: *mut c_int, first_bad: *mut i64, gt576: *mut u8) -> c_int;
+    // sets naming their message by index: one hash and one Miller pair per distinct message
+    pub fn b3_verify_multiple_grouped(ctx: *mut b3_ctx, t: *const b3_keytable, sigs192: *const u8, keys: *const c_void, pk_off: *const u32,
+                                      msgs: *const u8, msg_off: *const u32, n_msgs: usize, msg_idx: *const u32, scalars: *const u64,
+                                      n: usize, device_pointers: c_int, accept: *mut c_int, first_bad: *mut i64, gt576: *mut u8) -> c_int;
     // per-set verdicts after a rejected whole verify_multiple call on the same context
     pub fn b3_verify_multiple_locate(ctx: *mut b3_ctx, n: usize, valid: *mut i32, n_invalid: *mut usize) -> c_int;
     // two-phase form: the RNG contract of M/aggregates.rs:272-287 without running the subgroup checks twice
