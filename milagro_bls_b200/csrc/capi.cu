@@ -12,6 +12,7 @@
 #include <condition_variable>
 #include <mutex>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/milagro_bls_b200.h"
@@ -25,7 +26,7 @@ static const size_t kDstG2Len = 43;
 
 #define B3_MAX_MARKS 24
 // sets from which the key aggregation uses 4 lanes per set instead of 8 (less shuffle-tree overhead, twice the latency)
-static const size_t kAggG4Min = getenv("B3_AGG_G4_MIN") ? (size_t)atol(getenv("B3_AGG_G4_MIN")) : 4096;
+static const size_t kAggG4Min = 4096;
 #define B3_MSM_MIN_SETS 512     // below this, S = sum [c_j] sig_j uses n separate ladders + a tree
 #define B3_N_STAGES 12
 // stage ids (b3_ctx_stage_ms / b3_stage_name)
@@ -115,6 +116,23 @@ static inline unsigned nblk(size_t n, int tpb = B3_TPB) { return (unsigned)((n +
         kern<<<(grid), (block), 0, (strm)>>>(__VA_ARGS__);   \
         ctx->launches++;                                     \
     } while (0)
+// A chain kernel over n items in the lane layout P, or in the replicated layout W when `wide` (quad.cuh): kern_of(L) is the
+// kernel's instantiation for layout L, which runs n << L::shift threads.
+template <class P, class W, class KernOf, class... A>
+static void launch_lanes(b3_ctx* ctx, cudaStream_t strm, bool wide, size_t n, KernOf kern_of, A... args) {
+    if (wide) LAUNCH_ON(strm, kern_of(W()), nblk(n << W::shift), B3_TPB, args...);
+    else LAUNCH_ON(strm, kern_of(P()), nblk(n << P::shift), B3_TPB, args...);
+}
+// An aggregation kernel over n_sets sets with G lanes per set: kern_of(std::integral_constant<int, G>) is its instantiation.
+// Enough lanes to fill the chip, few enough to keep the shuffle tree short (4 from g4_min sets: the tree runs at <= half the
+// lanes, so fewer lanes per set waste less).
+template <class KernOf, class... A>
+static void launch_agg(b3_ctx* ctx, cudaStream_t strm, size_t n_sets, size_t total_keys, size_t g4_min, KernOf kern_of, A... args) {
+    const size_t avg = total_keys / n_sets;
+    if (n_sets >= g4_min || avg <= 8) LAUNCH_ON(strm, kern_of(std::integral_constant<int, 4>()), nblk(n_sets * 4), B3_TPB, args...);
+    else if (n_sets >= 2048 || avg <= 32) LAUNCH_ON(strm, kern_of(std::integral_constant<int, 8>()), nblk(n_sets * 8), B3_TPB, args...);
+    else LAUNCH_ON(strm, kern_of(std::integral_constant<int, 32>()), nblk(n_sets * 32), B3_TPB, args...);
+}
 
 extern "C" void b3_ctx_destroy(b3_ctx* ctx);
 extern "C" int b3_ctx_create(int device, b3_ctx** out) {
@@ -301,10 +319,9 @@ static int g2_sum(b3_ctx* ctx, g2_jac* a, g2_jac* b, size_t n, g2_jac** res, cud
 static int miller_lines(b3_ctx* ctx, cudaStream_t strm, const g2_jac* q, size_t n_pairs, size_t first, size_t count, dev_buf& lines, dev_buf& qinf) {
     if (count == 0) return B3_OK;
     int sp = span_begin(ctx, count <= 64 && first > 0 ? ST_MILLER_LINES_SUMS : ST_MILLER_LINES, strm);   // the few pairs of the signature MSM are timed apart
-    if (ctx->wide_now || count <= 64)          // few pairs (the window sums of the signature MSM): always latency-bound
-        LAUNCH_ON(strm, k_miller_lines_q, nblk(4 * count), B3_TPB, q, n_pairs, first, count, (fp2*)lines.p, (uint32_t*)qinf.p);
-    else
-        LAUNCH_ON(strm, k_miller_lines, nblk(2 * count), B3_TPB, q, n_pairs, first, count, (fp2*)lines.p, (uint32_t*)qinf.p);
+    // few pairs (the window sums of the signature MSM): always latency-bound
+    launch_lanes<lanes_pair, lanes_quad>(ctx, strm, ctx->wide_now || count <= 64, count, [](auto L) { return k_miller_lines<decltype(L)>; },
+                                         q, n_pairs, first, count, (fp2*)lines.p, (uint32_t*)qinf.p);
     span_end(ctx, sp, strm);
     return B3_OK;
 }
@@ -410,21 +427,14 @@ static int first_status(b3_ctx* ctx, const int32_t* d_status, size_t n) {
     for (size_t i = 0; i < n; i++) if (h[i]) return h[i];
     return B3_OK;
 }
-// G1 key aggregation on `strm`.  Lanes per set: enough lanes to fill the chip, few enough to keep the shuffle tree short
-// (4 from kAggG4Min sets: the tree runs at <= half the lanes, so fewer lanes per set waste less).
+// G1 key aggregation on `strm`
 static int launch_g1_aggregate(b3_ctx* ctx, cudaStream_t strm, const uint8_t* d_pks, const uint32_t* d_off, size_t n_sets, size_t total_keys,
                                g1_jac* d_out, int32_t* d_status) {
     if (n_sets == 0) return B3_OK;
-    const size_t avg = total_keys / n_sets;
     const int chk = ctx->trusted ? 0 : 1;
-    if (n_sets >= kAggG4Min || avg <= 8) LAUNCH_ON(strm, k_g1_aggregate<4>, nblk(n_sets * 4), B3_TPB, d_pks, d_off, n_sets, d_out, d_status, chk);
-    else if (n_sets >= 2048 || avg <= 32) LAUNCH_ON(strm, k_g1_aggregate<8>, nblk(n_sets * 8), B3_TPB, d_pks, d_off, n_sets, d_out, d_status, chk);
-    else LAUNCH_ON(strm, k_g1_aggregate<32>, nblk(n_sets * 32), B3_TPB, d_pks, d_off, n_sets, d_out, d_status, chk);
+    launch_agg(ctx, strm, n_sets, total_keys, kAggG4Min, [](auto g) { return k_g1_aggregate<decltype(g)::value>; }, d_pks, d_off, n_sets, d_out,
+               d_status, chk);
     return B3_OK;
-}
-static int g1_aggregate_dev_impl(b3_ctx* ctx, const uint8_t* d_pks, const uint32_t* d_off, size_t n_sets, size_t total_keys,
-                                 g1_jac* d_out, int32_t* d_status) {
-    return launch_g1_aggregate(ctx, ctx->stream, d_pks, d_off, n_sets, total_keys, d_out, d_status);
 }
 
 // ---------------------------------------------------------------------------------------------- serialisation API
@@ -499,7 +509,7 @@ extern "C" int b3_g2_subgroup_check(b3_ctx* ctx, const uint8_t* in192, size_t n,
     CKR(ensure(ctx, ctx->status, 4 * n));
     CKR(ensure(ctx, ctx->ok, 4 * n));
     LAUNCH(k_g2_parse, nblk(n), B3_TPB, (const uint8_t*)ctx->in_a.p, n, (g2_aff*)ctx->g2a_sig.p, (int32_t*)ctx->status.p, 1);
-    LAUNCH(k_g2_subgroup, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)ctx->status.p, n, (int32_t*)ctx->ok.p);
+    LAUNCH(k_g2_subgroup<lanes_pair>, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)ctx->status.p, n, (int32_t*)ctx->ok.p);
     CKR(d2h(ctx, status, ctx->status.p, 4 * n));
     CKR(d2h(ctx, ok, ctx->ok.p, 4 * n));
     return sync(ctx);
@@ -517,7 +527,7 @@ extern "C" int b3_g1_aggregate_dev(b3_ctx* ctx, const uint8_t* pks96_dev, const 
     uint32_t total = 0;
     CK(cudaMemcpyAsync(&total, off_dev + n_sets, 4, cudaMemcpyDeviceToHost, ctx->stream));
     CKR(sync(ctx));
-    CKR(g1_aggregate_dev_impl(ctx, pks96_dev, off_dev, n_sets, total, (g1_jac*)ctx->g1j.p, status_dev));
+    CKR(launch_g1_aggregate(ctx, ctx->stream, pks96_dev, off_dev, n_sets, total, (g1_jac*)ctx->g1j.p, status_dev));
     LAUNCH(k_g1_to_affine, nblk((n_sets + norm_per(n_sets) - 1) / norm_per(n_sets)), B3_TPB, (const g1_jac*)ctx->g1j.p, n_sets, (g1_aff*)ctx->g1a.p, norm_per(n_sets));
     LAUNCH(k_g1_aff_to_wire, nblk(n_sets), B3_TPB, (const g1_aff*)ctx->g1a.p, n_sets, out96_dev);
     return sync(ctx);
@@ -547,13 +557,9 @@ extern "C" int b3_g2_aggregate(b3_ctx* ctx, const uint8_t* sigs192, const uint32
     CKR(ensure(ctx, ctx->status, 4 * n_sets));
     CKR(ensure(ctx, ctx->g2j, sizeof(g2_jac) * n_sets));
     CKR(ensure(ctx, ctx->g2a, sizeof(g2_aff) * n_sets));
-    size_t avg = total / n_sets;
-    const uint8_t* d_in = (const uint8_t*)ctx->in_a.p;
-    const uint32_t* d_off = (const uint32_t*)ctx->in_b.p;
     const int chk = ctx->trusted ? 0 : 1;
-    if (n_sets >= 16384 || avg <= 8) LAUNCH(k_g2_aggregate<4>, nblk(n_sets * 4), B3_TPB, d_in, d_off, n_sets, (g2_jac*)ctx->g2j.p, (int32_t*)ctx->status.p, chk);
-    else if (n_sets >= 2048 || avg <= 32) LAUNCH(k_g2_aggregate<8>, nblk(n_sets * 8), B3_TPB, d_in, d_off, n_sets, (g2_jac*)ctx->g2j.p, (int32_t*)ctx->status.p, chk);
-    else LAUNCH(k_g2_aggregate<32>, nblk(n_sets * 32), B3_TPB, d_in, d_off, n_sets, (g2_jac*)ctx->g2j.p, (int32_t*)ctx->status.p, chk);
+    launch_agg(ctx, ctx->stream, n_sets, total, 16384, [](auto g) { return k_g2_aggregate<decltype(g)::value>; }, (const uint8_t*)ctx->in_a.p,
+               (const uint32_t*)ctx->in_b.p, n_sets, (g2_jac*)ctx->g2j.p, (int32_t*)ctx->status.p, chk);
     LAUNCH(k_g2_to_affine, nblk((n_sets + norm_per(n_sets) - 1) / norm_per(n_sets)), B3_TPB, (const g2_jac*)ctx->g2j.p, n_sets, (g2_aff*)ctx->g2a.p, norm_per(n_sets));
     LAUNCH(k_g2_aff_to_wire, nblk(n_sets), B3_TPB, (const g2_aff*)ctx->g2a.p, n_sets, (uint8_t*)ctx->outb.p);
     CKR(d2h(ctx, out192, ctx->outb.p, 192 * n_sets));
@@ -656,7 +662,7 @@ static int parse_sig(b3_ctx* ctx, const uint8_t* sig192) {
     CKR(ensure(ctx, ctx->status, 4 * 4));
     CKR(ensure(ctx, ctx->ok, 4 * 4));
     LAUNCH(k_g2_parse, 1, B3_TPB, (const uint8_t*)ctx->in_a.p, 1, (g2_aff*)ctx->g2a_sig.p, (int32_t*)ctx->status.p, 1);
-    LAUNCH(k_g2_subgroup, 1, B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)ctx->status.p, 1, (int32_t*)ctx->ok.p);
+    LAUNCH(k_g2_subgroup<lanes_pair>, 1, B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)ctx->status.p, 1, (int32_t*)ctx->ok.p);
     return first_status(ctx, (const int32_t*)ctx->status.p, 1);
 }
 extern "C" int b3_fast_aggregate_verify(b3_ctx* ctx, const uint8_t sig192[192], const uint8_t* pks96, size_t n_pks, const uint8_t* msg,
@@ -673,7 +679,7 @@ extern "C" int b3_fast_aggregate_verify(b3_ctx* ctx, const uint8_t sig192[192], 
     CKR(h2d(ctx, ctx->in_e, off, 8));
     CKR(ensure(ctx, ctx->g1j, sizeof(g1_jac) * 2));
     int32_t* d_st = (int32_t*)ctx->status.p + 1;
-    CKR(g1_aggregate_dev_impl(ctx, (const uint8_t*)ctx->in_b.p, (const uint32_t*)ctx->in_e.p, 1, n_pks, (g1_jac*)ctx->g1j.p, d_st));
+    CKR(launch_g1_aggregate(ctx, ctx->stream, (const uint8_t*)ctx->in_b.p, (const uint32_t*)ctx->in_e.p, 1, n_pks, (g1_jac*)ctx->g1j.p, d_st));
     CKR(first_status(ctx, d_st, 1));
     return verify_two_pairs(ctx, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)ctx->ok.p, (const g1_jac*)ctx->g1j.p, 1, msg, msg_len, accept, gt576);
 }
@@ -790,7 +796,7 @@ static int verify_batch_core(b3_ctx* ctx, int mode, const uint8_t* d_sigs, const
         CK(cudaStreamWaitEvent(s0, ctx->ev_fork2, 0));
     }
     sp = span_begin(ctx, ST_SIG_CHECK, s0);
-    LAUNCH_ON(s0, k_g2_subgroup, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)d_st_sig, n, (int32_t*)ctx->ok.p);
+    LAUNCH_ON(s0, k_g2_subgroup<lanes_pair>, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)d_st_sig, n, (int32_t*)ctx->ok.p);
     span_end(ctx, sp, s0);
     CKR(miller_lines(ctx, sm, q, 2 * n, 0, n, ctx->lines, ctx->qinf));
     // keys: aggregate (fast_aggregate_verify) or parse (verify / pre-aggregated) -> pairing form
@@ -954,13 +960,8 @@ extern "C" int b3_keytable_get(b3_ctx* ctx, const b3_keytable* t, const uint32_t
 static int launch_g1_aggregate_idx(b3_ctx* ctx, cudaStream_t strm, const b3_keytable* t, const uint32_t* d_idx, const uint32_t* d_off, size_t n_sets,
                                    size_t total_keys, g1_jac* d_out, int32_t* d_status) {
     if (n_sets == 0) return B3_OK;
-    const size_t avg = total_keys / n_sets;
-    if (n_sets >= kAggG4Min || avg <= 8)
-        LAUNCH_ON(strm, k_g1_aggregate_idx<4>, nblk(n_sets * 4), B3_TPB, (const key_entry*)t->d, t->n, d_idx, d_off, n_sets, d_out, d_status);
-    else if (n_sets >= 2048 || avg <= 32)
-        LAUNCH_ON(strm, k_g1_aggregate_idx<8>, nblk(n_sets * 8), B3_TPB, (const key_entry*)t->d, t->n, d_idx, d_off, n_sets, d_out, d_status);
-    else
-        LAUNCH_ON(strm, k_g1_aggregate_idx<32>, nblk(n_sets * 32), B3_TPB, (const key_entry*)t->d, t->n, d_idx, d_off, n_sets, d_out, d_status);
+    launch_agg(ctx, strm, n_sets, total_keys, kAggG4Min, [](auto g) { return k_g1_aggregate_idx<decltype(g)::value>; }, (const key_entry*)t->d,
+               t->n, d_idx, d_off, n_sets, d_out, d_status);
     return B3_OK;
 }
 // AggregatePublicKey::into_aggregate over table indices (M/src/aggregates.rs:46-56)
@@ -1110,15 +1111,14 @@ static int vm_stages(b3_ctx* ctx, const vm_in& in, size_t n_total, int32_t* d_st
     sp = span_begin(ctx, ST_G1_MUL, s1);
     if (in.d_msg_idx) {                   // [c_j] apk_j at the set's sorted position, a segmented tree per message, H_k's G1 member
         g1_jac* a = (g1_jac*)ctx->g1j2.p;
-        if (ctx->wide_now) LAUNCH_ON(s1, k_g1_mul_u64_jac_d, nblk(2 * n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, pos, n, a, d_zero);
-        else LAUNCH_ON(s1, k_g1_mul_u64_jac, nblk(n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, pos, n, a, d_zero);
+        launch_lanes<lanes_thread, lanes_pair>(ctx, s1, ctx->wide_now, n, [](auto L) { return k_g1_mul_u64<decltype(L), g1_out_at>; },
+                                               (const g1_jac*)ctx->g1j.p, in.d_scalars, n, g1_out_at{a, pos}, d_zero);
         for (size_t step = 1; step < n; step <<= 1)
             LAUNCH_ON(s1, k_grp_sum_level, nblk(n), B3_TPB, a, in.d_msg_idx, perm, lo, hi, n, m, step);
         LAUNCH_ON(s1, k_grp_to_pp, nblk(m), B3_TPB, (const g1_jac*)a, lo, hi, m, p);
-    } else if (ctx->wide_now) {
-        LAUNCH_ON(s1, k_g1_mul_u64_pp_d, nblk(2 * n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, n, p, d_zero);
     } else {
-        LAUNCH_ON(s1, k_g1_mul_u64_pp, nblk(n), B3_TPB, (const g1_jac*)ctx->g1j.p, in.d_scalars, n, p, d_zero);
+        launch_lanes<lanes_thread, lanes_pair>(ctx, s1, ctx->wide_now, n, [](auto L) { return k_g1_mul_u64<decltype(L), g1_out_pp>; },
+                                               (const g1_jac*)ctx->g1j.p, in.d_scalars, n, g1_out_pp{p}, d_zero);
     }
     span_end(ctx, sp, s1);
     // 5. S = sum_j [c_j] sig_j (M/src/aggregates.rs:303), on aux3: the context's own (highest-priority) stream is left to the
@@ -1167,10 +1167,9 @@ static int vm_sig_checks(b3_ctx* ctx, const vm_in& in, const int32_t* d_st_sig, 
     // the single CTA of the closing chain / final exponentiation (the replicated form fills every SM and halves their speed)
     const bool wide = ctx->wide_now && !in.defer_sig;
     int sp = span_begin(ctx, ST_SIG_CHECK, s0);
-    if (!in.prechecked) {
-        if (wide) LAUNCH_ON(s0, k_g2_subgroup_q, nblk(4 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, d_st_sig, n, (int32_t*)ctx->ok.p);
-        else LAUNCH_ON(s0, k_g2_subgroup, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, d_st_sig, n, (int32_t*)ctx->ok.p);
-    }
+    if (!in.prechecked)
+        launch_lanes<lanes_pair, lanes_quad>(ctx, s0, wide, n, [](auto L) { return k_g2_subgroup<decltype(L)>; }, (const g2_aff*)ctx->g2a_sig.p,
+                                             d_st_sig, n, (int32_t*)ctx->ok.p);
     LAUNCH_ON(s0, k_first_bad, nblk(n), B3_TPB, (const int32_t*)ctx->ok.p, n, in.index_base, d_first_bad);
     span_end(ctx, sp, s0);
     if (!ctx->serial) {
@@ -1445,7 +1444,7 @@ extern "C" int b3_sig_precheck(b3_ctx* ctx, const uint8_t* sigs192, size_t n, in
     ctx->h_init[0] = B3_FB_NONE;
     CK(cudaMemcpyAsync(d_fb, ctx->h_init, 8, cudaMemcpyHostToDevice, ctx->stream));
     LAUNCH(k_g2_parse, nblk(n), B3_TPB, (const uint8_t*)ctx->in_a.p, n, (g2_aff*)ctx->g2a_sig.p, (int32_t*)ctx->status.p, 1);
-    LAUNCH(k_g2_subgroup, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)ctx->status.p, n, (int32_t*)ctx->ok.p);
+    LAUNCH(k_g2_subgroup<lanes_pair>, nblk(2 * n), B3_TPB, (const g2_aff*)ctx->g2a_sig.p, (const int32_t*)ctx->status.p, n, (int32_t*)ctx->ok.p);
     LAUNCH(k_first_bad, nblk(n), B3_TPB, (const int32_t*)ctx->ok.p, n, 0LL, d_fb);
     CKR(first_status(ctx, (const int32_t*)ctx->status.p, n));          // malformed signature: the AmclError code
     long long fb = 0;

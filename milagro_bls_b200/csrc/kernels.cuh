@@ -45,29 +45,18 @@ __global__ void __launch_bounds__(B3_TPB) k_g2_parse(const uint8_t* __restrict__
     status[i] = e;
 }
 // subgroup_check_g2 on parsed signatures: ok[i] = parsed fine && in G2 (infinity passes, SURVEY.md C.4).
-// LANE PAIRS (fp2h.cuh): threads (2i, 2i+1) work on signature i.
+// L = lanes_pair or lanes_quad (quad.cuh)
+template <class L>
 __global__ void B3_LBH k_g2_subgroup(const g2_aff* pts, const int32_t* status, size_t n, int32_t* ok) {
-    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> L::shift;
     if (i >= n) return;
     int good = 0;
     if (status[i] == B3_OK) {
-        g2h_aff a;
-        g2h_load(a, pts[i]);
+        aff<typename L::g2> a;
+        L::load(a, pts[i]);
         good = g2_in_subgroup_aff(a) ? 1 : 0;
     }
-    if (!pair_odd()) ok[i] = good;
-}
-// the same on LANE QUADS (quad.cuh): threads 4i .. 4i+3 work on signature i, paired products split over the two lane pairs
-__global__ void B3_LBH k_g2_subgroup_q(const g2_aff* pts, const int32_t* status, size_t n, int32_t* ok) {
-    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 2;
-    if (i >= n) return;
-    int good = 0;
-    if (status[i] == B3_OK) {
-        g2q_aff a;
-        g2q_load(a, pts[i]);
-        good = g2_in_subgroup_aff(a) ? 1 : 0;
-    }
-    if ((threadIdx.x & 3u) == 0) ok[i] = good;
+    if (L::leader()) ok[i] = good;
 }
 // key_validate on parsed G1 points (not infinity, in G1)
 __global__ void __launch_bounds__(B3_TPB) k_g1_key_validate(const g1_jac* pts, const int32_t* status, size_t n, int32_t* valid) {
@@ -319,6 +308,27 @@ __device__ __forceinline__ void shfl_down_struct(P& dst, const P& src, int delta
 #pragma unroll 1
     for (int k = 0; k < (int)(sizeof(P) / 4); k++) d[k] = __shfl_down_sync(0xffffffffu, s[k], delta, width);
 }
+// The shuffle tree of a group (lane = its lane in the group, the sum and the status of the group end in lane 0), then lane 0
+// of an active group stores them: status = the error of some failing lane, else B3_ERR_AGGREGATE_EMPTY_POINTS_D when
+// `empty`, else 0.
+template <int G, class P>
+__device__ __forceinline__ void agg_tree_store(P& acc, int err, int lane, bool active, bool empty, P* out, int32_t* status, size_t gid) {
+#pragma unroll 1
+    for (int d = G / 2; d >= 1; d >>= 1) {
+        P o;
+        shfl_down_struct(o, acc, d, G);
+        int oe = __shfl_down_sync(0xffffffffu, err, d, G);
+        if (lane < d) {
+            pt_add(acc, acc, o);
+            if (oe) err = oe;
+        }
+    }
+    if (active && lane == 0) {
+        if (empty) err = B3_ERR_AGGREGATE_EMPTY_POINTS_D;
+        out[gid] = acc;
+        status[gid] = err;
+    }
+}
 
 // The keys are the bulk of the input bytes (C4: 100 MB of 103 MB), so they are STAGED: the G lanes of a group fetch the group's
 // next run of G consecutive 96-byte records as 16-byte words, lane l taking words l, l + G, ... (LDG.128, each warp request
@@ -373,21 +383,7 @@ __global__ void __launch_bounds__(B3_TPB) k_g1_aggregate(const uint8_t* __restri
         }
     }
 #undef B3_AGG_FETCH
-#pragma unroll 1
-    for (int d = G / 2; d >= 1; d >>= 1) {
-        g1_jac o;
-        shfl_down_struct(o, acc, d, G);
-        int oe = __shfl_down_sync(0xffffffffu, err, d, G);
-        if (lane < d) {
-            pt_add(acc, acc, o);
-            if (oe) err = oe;
-        }
-    }
-    if (active && lane == 0) {
-        if (b == e) err = B3_ERR_AGGREGATE_EMPTY_POINTS_D;
-        out[gid] = acc;
-        status[gid] = err;
-    }
+    agg_tree_store<G>(acc, err, lane, active, b == e, out, status, gid);
 }
 // The same aggregation over a device-resident key table: set s owns the table entries idx[off[s] .. off[s+1]).  A gather of
 // 96-byte entries (three full 32-byte sectors each), the next entry in flight while the current one is added.
@@ -425,21 +421,7 @@ __global__ void __launch_bounds__(B3_TPB) k_g1_aggregate_idx(const key_entry* __
         else pt_add_aff(acc, acc, a);
         cur = nxt; ok = okn; have = hn; i = inext;
     }
-#pragma unroll 1
-    for (int d = G / 2; d >= 1; d >>= 1) {
-        g1_jac o;
-        shfl_down_struct(o, acc, d, G);
-        int oe = __shfl_down_sync(0xffffffffu, err, d, G);
-        if (lane < d) {
-            pt_add(acc, acc, o);
-            if (oe) err = oe;
-        }
-    }
-    if (active && lane == 0) {
-        if (b == e) err = B3_ERR_AGGREGATE_EMPTY_POINTS_D;
-        out[gid] = acc;
-        status[gid] = err;
-    }
+    agg_tree_store<G>(acc, err, lane, active, b == e, out, status, gid);
 }
 // G2 aggregation (AggregateSignature::aggregate): same shape over Fp2 (records read as 12 x LDG.128 per lane)
 template <int G>
@@ -460,20 +442,7 @@ __global__ void __launch_bounds__(B3_TPB) k_g2_aggregate(const uint8_t* __restri
         if (s) err = s;
         else pt_add_aff(acc, acc, a);
     }
-#pragma unroll 1
-    for (int d = G / 2; d >= 1; d >>= 1) {
-        g2_jac o;
-        shfl_down_struct(o, acc, d, G);
-        int oe = __shfl_down_sync(0xffffffffu, err, d, G);
-        if (lane < d) {
-            pt_add(acc, acc, o);
-            if (oe) err = oe;
-        }
-    }
-    if (active && lane == 0) {
-        out[gid] = acc;
-        status[gid] = err;
-    }
+    agg_tree_store<G>(acc, err, lane, active, false, out, status, gid);
 }
 
 // ------------------------------------------------------------------------------------------------ scalar multiplication
@@ -843,47 +812,44 @@ __global__ void __launch_bounds__(B3_TPB) k_g1_jac_to_pp(const g1_jac* in, size_
     g1_pp_from_jac(r, p);
     out[i] = r;
 }
-// P_j = [c_j] apk_j straight into pairing form
+// P_j = [c_j] apk_j on L = lanes_thread or lanes_pair (quad.cuh), written by Out:
+//   g1_out_pp: in pairing form at j (the pair member of set j)
+//   g1_out_at: Jacobian at pos[j] (grouped calls: the set's sorted position, see below)
 // zero_flag: set when a scalar is 0 -- the reference's draw rule never yields 0 (M/src/aggregates.rs:280-286), and a zero scalar
 // would drop its set from the batch equation, so the call is rejected (B3_ERR_ARG)
-__global__ void __launch_bounds__(B3_TPB) k_g1_mul_u64_pp(const g1_jac* in, const uint64_t* __restrict__ k, size_t n, g1_pp* out, int32_t* zero_flag) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+struct g1_out_pp {
+    g1_pp* out;
+    template <class L>
+    __device__ __forceinline__ void put(size_t i, const jac<typename L::g1>& r) const {
+        g1_pp o;
+        g1_pp_from_jac(o, r);
+        if (L::leader()) out[i] = o;
+    }
+};
+struct g1_out_at {
+    g1_jac* out;
+    const uint32_t* pos;
+    template <class L>
+    __device__ __forceinline__ void put(size_t i, const jac<typename L::g1>& r) const {
+        if (L::leader()) L::store(out[__ldg(pos + i)], r);
+    }
+};
+template <class L, class Out>
+__global__ void __launch_bounds__(B3_TPB) k_g1_mul_u64(const g1_jac* in, const uint64_t* __restrict__ k, size_t n, Out out, int32_t* zero_flag) {
+    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> L::shift;
     if (i >= n) return;
-    g1_jac p = in[i], r;
-    if (k[i] == 0) *zero_flag = 1;
-    pt_mul_u64_w4(r, p, k[i]);
-    g1_pp o;
-    g1_pp_from_jac(o, r);
-    out[i] = o;
-}
-// the same on LANE PAIRS (quad.cuh: fpd): threads (2i, 2i+1) work on set i, the paired products of the point formulas split
-// over the two lanes
-__global__ void __launch_bounds__(B3_TPB) k_g1_mul_u64_pp_d(const g1_jac* in, const uint64_t* __restrict__ k, size_t n, g1_pp* out, int32_t* zero_flag) {
-    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
-    if (i >= n) return;
-    g1d_jac p, r;
-    g1d_load(p, in[i]);
+    jac<typename L::g1> p, r;
+    L::load(p, in[i]);
     const uint64_t c = k[i];
     if (c == 0) *zero_flag = 1;
     pt_mul_u64_w4(r, p, c);
-    // pairing form (X Z, -Y, Z^3): Z^2 and X Z as a pair, then Z^3
-    fpd z2, xz, z3;
-    f_mulsqr_par(xz, r.x, r.z, z2, r.z);
-    f_mul(z3, z2, r.z);
-    if (!pair_odd()) {
-        g1_pp o;
-        o.xz = xz.v;
-        fp_neg(o.ny, r.y.v);
-        o.z3 = z3.v;
-        o.inf = fp_is_zero(r.z.v) ? 1u : 0u;
-        out[i] = o;
-    }
+    out.template put<L>(i, r);
 }
 
 // ---- sets grouped by message (b3_verify_multiple_grouped) --------------------------------------------------------------
 // By bilinearity prod_(j in g) e([c_j] apk_j, H(m)) = e(sum_(j in g) [c_j] apk_j, H(m)): the sets naming message k share one
 // pair, whose G1 member is the sum of their scaled keys.  The set indices are sorted by message (k_grp_sort), each set's
-// [c_j] apk_j is written at its sorted position (k_g1_mul_u64_jac*), and every message's run of positions is reduced by a
+// [c_j] apk_j is written at its sorted position (k_g1_mul_u64 with g1_out_at), and every message's run of positions is reduced by a
 // segmented pairwise tree (k_grp_sum_level, one launch per level: log2(n) levels whatever the group sizes).
 // An out-of-range message index raises the flag and is read as message 0, so nothing indexes past the tables (the call is
 // then rejected).
@@ -954,32 +920,6 @@ __global__ void __launch_bounds__(B3_TPB) k_grp_bounds(const uint32_t* __restric
     if (i == 0 || grp_key(key, perm[i - 1], m) != k) lo[k] = (uint32_t)i;
     if (i + 1 == n || grp_key(key, perm[i + 1], m) != k) hi[k] = (uint32_t)(i + 1);
 }
-// P_j = [c_j] apk_j, Jacobian, at the sorted position pos[j]; zero_flag as in k_g1_mul_u64_pp
-__global__ void __launch_bounds__(B3_TPB) k_g1_mul_u64_jac(const g1_jac* in, const uint64_t* __restrict__ k, const uint32_t* __restrict__ pos, size_t n,
-                                                           g1_jac* out, int32_t* zero_flag) {
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    g1_jac p = in[i], r;
-    if (k[i] == 0) *zero_flag = 1;
-    pt_mul_u64_w4(r, p, k[i]);
-    out[pos[i]] = r;
-}
-// the same on LANE PAIRS (the latency mode, as k_g1_mul_u64_pp_d)
-__global__ void __launch_bounds__(B3_TPB) k_g1_mul_u64_jac_d(const g1_jac* in, const uint64_t* __restrict__ k, const uint32_t* __restrict__ pos, size_t n,
-                                                             g1_jac* out, int32_t* zero_flag) {
-    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
-    if (i >= n) return;
-    g1d_jac p, r;
-    g1d_load(p, in[i]);
-    const uint64_t c = k[i];
-    if (c == 0) *zero_flag = 1;
-    pt_mul_u64_w4(r, p, c);
-    if (!pair_odd()) {
-        g1_jac o;
-        o.x = r.x.v; o.y = r.y.v; o.z = r.z.v;
-        out[pos[i]] = o;
-    }
-}
 // one level of the segmented tree: inside each message's run [lo, hi), position lo + r with r % (2 step) == 0 adds in position
 // lo + r + step.  After the levels step = 1, 2, 4, .. < n, position lo[k] holds the sum of the run (pt_add: complete, so
 // equal points -- one key and one scalar twice in a group -- and opposite points are exact).
@@ -1026,74 +966,32 @@ __global__ void __launch_bounds__(B3_TPB) k_g2_aff_to_jac(const g2_aff* in, size
 
 // ---- split multi-Miller loop (pairing.cuh: "split Miller loop") ---------------------------------------------------
 // 1. point chain of every pair -> unscaled lines, lines[(slot * n + pair) * 3 + {0,1,2}] = (u0, l3, u5)
-//    LANE PAIRS: threads (2i, 2i+1) run the chain of pair i, each storing its half of every coefficient.
+//    L = lanes_pair or lanes_quad (quad.cuh): the lanes of pair i run its chain and store the coefficients of every line.
 //    Pairs [first, first + count) of the n pairs of the product (different ranges may run on different streams).
+template <class L>
 __global__ void B3_LBH k_miller_lines(const g2_jac* __restrict__ q, size_t n, size_t first, size_t count,
-                                                         fp2* __restrict__ lines, uint32_t* __restrict__ qinf) {
-    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 1;
+                                      fp2* __restrict__ lines, uint32_t* __restrict__ qinf) {
+    typedef typename L::g2 F2;
+    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> L::shift;
     if (i >= count) return;
     i += first;
-    fp2h X, Y, Z;
-    fp2h_load(X, q[i].x);
-    fp2h_load(Y, q[i].y);
-    fp2h_load(Z, q[i].z);
-    const bool inf = fp2_is_zero(Z);
-    if (!pair_odd()) qinf[i] = inf ? 1u : 0u;
+    jac<F2> p;
+    L::load(p, q[i]);
+    const bool inf = fp2_is_zero(p.z);
+    if (L::leader()) qinf[i] = inf ? 1u : 0u;
     if (inf) return;                           // its lines are never read: the accumulate kernel skips the pair
-    miller_pt_t<fp2h> t, Q;
-    miller_start(t, X, Y, Z);
+    miller_pt_t<F2> t, Q;
+    miller_start(t, p.x, p.y, p.z);
     Q = t;
     const uint64_t x = B3_X_ABS;
     int a = B3_MILLER_DBL_SLOTS;
-    fp2h u0, l3, u5;
+    F2 u0, l3, u5;
     for (int it = 0; it < B3_MILLER_DBL_SLOTS; it++) {
         miller_dbl_step_u(t, u0, l3, u5);
-        fp2* o = lines + ((size_t)it * n + i) * 3;
-        fp2h_store(o[0], u0); fp2h_store(o[1], l3); fp2h_store(o[2], u5);
+        L::store_line(lines + ((size_t)it * n + i) * 3, u0, l3, u5);
         if ((x >> (62 - it)) & 1) {
             miller_add_step_u(t, u0, l3, u5, Q.x, Q.y, Q.z);
-            o = lines + ((size_t)a * n + i) * 3;
-            fp2h_store(o[0], u0); fp2h_store(o[1], l3); fp2h_store(o[2], u5);
-            a++;
-        }
-    }
-}
-//    LANE QUADS (quad.cuh): threads 4i .. 4i+3 run the chain of pair i with the paired products of every step split over
-//    the two lane pairs; the low pair stores u0 and l3, the high pair u5.
-__global__ void B3_LBH k_miller_lines_q(const g2_jac* __restrict__ q, size_t n, size_t first, size_t count,
-                                        fp2* __restrict__ lines, uint32_t* __restrict__ qinf) {
-    size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 2;
-    if (i >= count) return;
-    i += first;
-    fp2q X, Y, Z;
-    fp2h_load(X, q[i].x);
-    fp2h_load(Y, q[i].y);
-    fp2h_load(Z, q[i].z);
-    const bool inf = fp2_is_zero(Z);
-    if ((threadIdx.x & 3u) == 0) qinf[i] = inf ? 1u : 0u;
-    if (inf) return;                           // its lines are never read: the accumulate kernel skips the pair
-    miller_pt_t<fp2q> t, Q;
-    {                                          // homogeneous (X Z : Y : Z^3)
-        fp2q z2;
-        f_mulsqr_par(t.x, X, Z, z2, Z);
-        t.y = Y;
-        f_mul(t.z, z2, Z);
-    }
-    Q = t;
-    const uint64_t x = B3_X_ABS;
-    const bool hi = quad_hi();
-    int a = B3_MILLER_DBL_SLOTS;
-    fp2q u0, l3, u5;
-    for (int it = 0; it < B3_MILLER_DBL_SLOTS; it++) {
-        miller_dbl_step_u(t, u0, l3, u5);
-        fp2* o = lines + ((size_t)it * n + i) * 3;
-        if (hi) fp2h_store(o[2], u5);
-        else { fp2h_store(o[0], u0); fp2h_store(o[1], l3); }
-        if ((x >> (62 - it)) & 1) {
-            miller_add_step_u(t, u0, l3, u5, Q.x, Q.y, Q.z);
-            o = lines + ((size_t)a * n + i) * 3;
-            if (hi) fp2h_store(o[2], u5);
-            else { fp2h_store(o[0], u0); fp2h_store(o[1], l3); }
+            L::store_line(lines + ((size_t)a * n + i) * 3, u0, l3, u5);
             a++;
         }
     }

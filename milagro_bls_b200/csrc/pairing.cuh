@@ -87,10 +87,9 @@ B3_FN_NOINLINE void miller_add_step_u(miller_pt_t<F2>& t, F2& u0, F2& l3, F2& u5
 template <class F2>
 B3_FN void miller_start(miller_pt_t<F2>& t, const F2& X, const F2& Y, const F2& Z) {
     F2 z2;
-    fp2_sqr(z2, Z);
-    fp2_mul(t.x, X, Z);
+    f_mulsqr_par(t.x, X, Z, z2, Z);
     t.y = Y;
-    fp2_mul(t.z, z2, Z);
+    f_mul(t.z, z2, Z);
 }
 // G1 member of a pairing in the form the line scaling wants: for P = (X : Y : Z) Jacobian (x = X/Z^2, y = Y/Z^3)
 // the line  l0 = u0 (-y), l3, l5 = u5 x  times Z^3 is  u0 (-Y), l3 Z^3, u5 (X Z)  -- no inversion.
@@ -98,12 +97,16 @@ struct g1_pp {
     fp xz, ny, z3;
     uint32_t inf;
 };
-B3_FN void g1_pp_from_jac(g1_pp& r, const g1_jac& p) {
-    fp z2;
-    fp_sqr(z2, p.z);
-    fp_mul(r.xz, p.x, p.z);
-    fp_neg(r.ny, p.y);
-    fp_mul(r.z3, z2, p.z);
+// P in any G1 representation whose lanes each hold the whole value (fp; fpd, quad.cuh)
+B3_FN const fp& fp_of(const fp& a) { return a; }
+template <class F>
+B3_FN void g1_pp_from_jac(g1_pp& r, const jac<F>& p) {
+    F xz, z2, z3;
+    f_mulsqr_par(xz, p.x, p.z, z2, p.z);
+    f_mul(z3, z2, p.z);
+    r.xz = fp_of(xz);
+    fp_neg(r.ny, fp_of(p.y));
+    r.z3 = fp_of(z3);
     r.inf = pt_is_inf(p) ? 1u : 0u;
 }
 

@@ -11,8 +11,9 @@
 //   G1/G2 doubling (2M + 5S)    : 4 rounds instead of 7 products        G2 mixed addition (7M + 4S): 6 instead of 11
 //   Miller doubling step (3M+6S): 5 rounds instead of 9                 Miller addition step (16M + 2S): 9 instead of 18
 // A squaring paired with a multiplication runs as a multiplication (both halves of a warp execute one instruction stream).
-// The replicated kernels do ~25 % more multiply-accumulates than the plain ones, so they are used only when a call cannot
-// fill the GPU by itself (capi.cu: latency_mode).
+// The chain kernels are templates over the lane layouts at the end of this file.  Their replicated instantiations
+// (lanes_pair for G1, lanes_quad for G2) do ~25 % more multiply-accumulates than the plain ones (lanes_thread, lanes_pair),
+// so they run only when a call cannot fill the GPU by itself (capi.cu: latency_mode).
 #pragma once
 #include "fp2h.cuh"
 
@@ -33,6 +34,7 @@ B3_FN void f_select(fpd& r, bool c, const fpd& a, const fpd& b) { fp_select(r.v,
 B3_FN void f_one(fpd& r) { r.v = FP_ONE; }
 B3_FN void f_zero(fpd& r) { r.v = FP_NIL; }
 B3_FN void f_mul_b(fpd& r, const fpd& a) { fp t; fp_dbl(t, a.v); fp_dbl(r.v, t); }
+B3_FN const fp& fp_of(const fpd& a) { return a.v; }      // every lane holds the whole value
 // the odd lane takes the second product of the pair
 B3_FN void f_mul_par(fpd& r1, const fpd& a1, const fpd& b1, fpd& r2, const fpd& a2, const fpd& b2) {
     const bool odd = pair_odd();
@@ -63,8 +65,6 @@ B3_FN void f_mulsqr_par(fpd& r1, const fpd& a1, const fpd& b1, fpd& r2, const fp
     fp_select(r1.v, odd, o, p);
     fp_select(r2.v, odd, p, o);
 }
-typedef jac<fpd> g1d_jac;
-__device__ __forceinline__ void g1d_load(g1d_jac& r, const g1_jac& a) { r.x.v = a.x; r.y.v = a.y; r.z.v = a.z; }
 
 // ---------------------------------------------------------------------------------------------- fp2q: Fp2 on a lane quad
 // lane l of the quad: half (l & 1) of the Fp2 value as in fp2h, in pair (l >> 1) & 1.  Every fp2h routine applies unchanged
@@ -110,12 +110,44 @@ B3_FN void f_mulsqr_par(fp2q& r1, const fp2q& a1, const fp2q& b1, fp2q& r2, cons
     fp_select(r1.v, hi, o, p.v);
     fp_select(r2.v, hi, p.v, o);
 }
-typedef jac<fp2q> g2q_jac;
-typedef aff<fp2q> g2q_aff;
-__device__ __forceinline__ void g2q_load(g2q_jac& r, const g2_jac& a) { fp2h_load(r.x, a.x); fp2h_load(r.y, a.y); fp2h_load(r.z, a.z); }
-__device__ __forceinline__ void g2q_load(g2q_aff& r, const g2_aff& a) { fp2h_load(r.x, a.x); fp2h_load(r.y, a.y); r.inf = a.inf; }
-// only the low pair of the quad stores
-__device__ __forceinline__ void g2q_store(g2_jac& a, const g2q_jac& r) {
-    if (!quad_hi()) { fp2h_store(a.x, r.x); fp2h_store(a.y, r.y); fp2h_store(a.z, r.z); }
-}
+// ---------------------------------------------------------------------------------------------- lane layouts
+// The chain kernels (kernels.cuh) are templates over a lane layout L: item i runs on the 1 << L::shift lanes from
+// i << L::shift, holding its G1 values as L::g1 and its G2 values as L::g2.  L::leader() is the one lane of the group that
+// writes a single-writer result; L::load / L::store convert between a full point in memory and the group's values.
+//   lanes_thread: one thread per item (G1 in fp)
+//   lanes_pair  : G1 replicated in fpd, G2 split over the pair in fp2h (fp2h.cuh)
+//   lanes_quad  : G2 replicated in fp2q
+struct lanes_thread {
+    typedef fp g1;
+    static constexpr unsigned shift = 0;
+    static __device__ __forceinline__ bool leader() { return true; }
+    static __device__ __forceinline__ void load(g1_jac& r, const g1_jac& a) { r = a; }
+    static __device__ __forceinline__ void store(g1_jac& a, const g1_jac& r) { a = r; }
+};
+struct lanes_pair {
+    typedef fpd g1;
+    typedef fp2h g2;
+    static constexpr unsigned shift = 1;
+    static __device__ __forceinline__ bool leader() { return !pair_odd(); }
+    static __device__ __forceinline__ void load(jac<fpd>& r, const g1_jac& a) { r.x.v = a.x; r.y.v = a.y; r.z.v = a.z; }
+    static __device__ __forceinline__ void store(g1_jac& a, const jac<fpd>& r) { a.x = r.x.v; a.y = r.y.v; a.z = r.z.v; }
+    static __device__ __forceinline__ void load(g2h_jac& r, const g2_jac& a) { g2h_load(r, a); }
+    static __device__ __forceinline__ void load(g2h_aff& r, const g2_aff& a) { g2h_load(r, a); }
+    // the coefficients (u0, l3, u5) of a Miller line at o: each lane stores its half of all three
+    static __device__ __forceinline__ void store_line(fp2* o, const fp2h& u0, const fp2h& l3, const fp2h& u5) {
+        fp2h_store(o[0], u0); fp2h_store(o[1], l3); fp2h_store(o[2], u5);
+    }
+};
+struct lanes_quad {
+    typedef fp2q g2;
+    static constexpr unsigned shift = 2;
+    static __device__ __forceinline__ bool leader() { return (threadIdx.x & 3u) == 0; }
+    static __device__ __forceinline__ void load(jac<fp2q>& r, const g2_jac& a) { fp2h_load(r.x, a.x); fp2h_load(r.y, a.y); fp2h_load(r.z, a.z); }
+    static __device__ __forceinline__ void load(aff<fp2q>& r, const g2_aff& a) { fp2h_load(r.x, a.x); fp2h_load(r.y, a.y); r.inf = a.inf; }
+    // the low pair stores u0 and l3, the high pair u5
+    static __device__ __forceinline__ void store_line(fp2* o, const fp2q& u0, const fp2q& l3, const fp2q& u5) {
+        if (quad_hi()) fp2h_store(o[2], u5);
+        else { fp2h_store(o[0], u0); fp2h_store(o[1], l3); }
+    }
+};
 #endif
