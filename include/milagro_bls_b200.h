@@ -93,7 +93,8 @@ int b3_g1_aggregate(b3_ctx*, const uint8_t* pks96, const uint32_t* off, size_t n
 int b3_g2_aggregate(b3_ctx*, const uint8_t* sigs192, const uint32_t* off, size_t n_sets, uint8_t* out192, int32_t* status);
 
 /* ---- hash_to_curve_g2 (M/src/amcl_utils.rs:33-35 -> A/bls381/core.rs:831-839).  Message i is
- *      msgs[off[i] .. off[i+1]).  dst == NULL selects DST_G2 (A/bls381/proof_of_possession.rs:38). */
+ *      msgs[off[i] .. off[i+1]).  dst == NULL selects DST_G2 (A/bls381/proof_of_possession.rs:38).  Any other DST may hold
+ *      0 to 255 bytes; a longer one returns B3_ERR_HASH_TO_FIELD and hashes nothing (milagro_bls never passes one). */
 int b3_hash_to_g2(b3_ctx*, const uint8_t* msgs, const uint32_t* off, size_t n, const uint8_t* dst, size_t dst_len,
                   uint8_t* out192);
 
